@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the hot path: Fr gate evals/sec, range_check batch 2^24 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--log2n 24] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--log2n 24] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic witnesses:
     fresh composer -> add_input(2^log2n witnesses) -> range_check(0, 2^64) [witness generation: 271 rows / 653 variables
@@ -14,6 +14,8 @@ Multi-GPU: one process per GPU (torchrun), instances sharded by pg_shard_plan (w
 2^log2n in total), the only collective of the step is the all-reduce of the verdict (pg_check_sharded: NCCL through the C ABI),
 executed inside every timed step.  `--impl reference` times the restated reference CPU path (oracle/, faithful cost
 structure: per-bit 256-step pow, hash-map variable store, per-row column pushes) on all host cores, rank 0 only.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step computed as .npy files (dump_outputs below), so
+that two builds can be compared output for output: the synthetic witnesses depend only on the arguments.
 """
 from __future__ import annotations
 
@@ -27,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "Fr gate evals/sec, range_check batch 2^24"
 UNIT = "gate-evals/s"
@@ -185,6 +188,42 @@ def bind_to_gpu_numa_node(index: int):
     return None
 
 
+DUMP_SEED = 0x64756D70           # the sampled instances depend only on the batch size: the same files on every run
+DUMP_RESULTS = 1 << 18           # instances whose range_check result is written (16 MiB)
+DUMP_BLOCKS = 256                # instances whose whole variable block (VARS_PER_INSTANCE Fr each) is written (10.7 MB)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def fr_words(a):
+    """(..., 4) uint64 Fr limbs as the C ABI returns them (Montgomery form) -> (..., 8) float64 of their little-endian 32-bit words,
+    which float64 holds exactly."""
+    import numpy as np
+    a = np.ascontiguousarray(a, dtype=np.uint64)
+    return a.view(np.uint32).reshape(a.shape[:-1] + (8,)).astype(np.float64)
+
+
+def dump_outputs(out_dir: str, c, res, n: int, bad: int, first):
+    """What the last timed step handed its caller, as float64 .npy files in out_dir:
+      range_check_results[_index]    the result column y (res: all n results of this rank, on the device) at a seeded sample of instances
+      variables[_index]              the witness generation's variable block of a smaller seeded sample of instances: (m, 653, 8)
+      verdict                        [unsatisfied rows, first unsatisfied row or -1] of the whole batch"""
+    import numpy as np
+    import torch
+    rng = np.random.default_rng(DUMP_SEED)
+    idx = np.sort(rng.choice(n, min(n, DUMP_RESULTS), replace=False))
+    blk = np.sort(rng.choice(n, min(n, DUMP_BLOCKS), replace=False))
+    results = res[torch.from_numpy(idx).to(res.device)].cpu().numpy().view(np.uint64)
+    base = c.num_variables() - VARS_PER_INSTANCE * n                 # range_check allocates one block of VARS_PER_INSTANCE per instance, last
+    blocks = np.stack([c.variables(base + VARS_PER_INSTANCE * int(i), VARS_PER_INSTANCE) for i in blk])
+    arrays = {"range_check_results": fr_words(results), "range_check_results_index": idx.astype(np.float64),
+              "variables": fr_words(blocks), "variables_index": blk.astype(np.float64),
+              "verdict": np.array([bad, -1 if first is None else first], dtype=np.float64)}
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _JSON_FD = None
 
 
@@ -217,7 +256,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--check-shape", type=int, default=0, help="launch shape of the gate-check kernel (tuning knob)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="weak: 2^log2n instances per GPU; strong: 2^log2n in total")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0's instances) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs: not with --impl reference")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -314,6 +358,8 @@ def main():
     c.read_column_into(y, res); c.sync()
     one_t = torch.from_numpy(one_limbs.view(np.int64)).to(dev)
     assert bool((res[0::2] == one_t).all()) and bool((res[1::2] == 0).all()) and tot_bad == 0, "result pattern / verdict"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, c, res, n, bad, first)
 
     # e2e (host buffers, copies inside the timed region)
     for _ in range(2):

@@ -7,8 +7,11 @@
 // satisfies the gate equation", which is equivalent for these circuits (copy constraints hold by construction).
 // All cases of one test are batched into ONE gadget call (one instance per case).  Exit code 0 = all verdicts as expected.
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
+#include <string>
 #include <vector>
+#include <unistd.h>
 #include "plonk_gadgets.hpp"
 
 using namespace plonk_gadgets;
@@ -217,11 +220,19 @@ static void batch_extensions_test() {
         EXPECT(all == composer.values(res) && all[0] == BlsScalar::one() && all[1] == BlsScalar::zero(), "gathered results");
         const uint64_t vars_per = 2 * 19 + 523;
         EXPECT(composer.gather_variables(1, 300 * vars_per) == composer.variables(5 + 300, 300 * vars_per), "gathered witness shard == the composer's variables");
-        composer.export_to("/tmp/pg_cpp_mirror_export.pgexp", true);
-        FILE* f = std::fopen("/tmp/pg_cpp_mirror_export.pgexp", "rb");
+        // a file of this run's own: a fixed name would collide with (or be left unwritable by) another user's run on the same host
+        const char* tmpdir = std::getenv("TMPDIR");
+        std::string path = std::string(tmpdir && *tmpdir ? tmpdir : "/tmp") + "/pg_cpp_mirror_export_XXXXXX";
+        const int fd = mkstemp(&path[0]);
+        EXPECT(fd >= 0, "temporary export file");
+        if (fd < 0) continue;
+        close(fd);
+        composer.export_to(path, true);
+        FILE* f = std::fopen(path.c_str(), "rb");
         char magic[8] = {0}; uint32_t ver = 0, flags = 0; uint64_t head[3] = {0, 0, 0};
         const bool read_ok = f && std::fread(magic, 1, 8, f) == 8 && std::fread(&ver, 4, 1, f) == 1 && std::fread(&flags, 4, 1, f) == 1 && std::fread(head, 8, 3, f) == 3;
         if (f) std::fclose(f);
+        std::remove(path.c_str());
         EXPECT(read_ok && std::memcmp(magic, "PGB2EXP1", 8) == 0 && ver == 1 && flags == 1 && head[0] == composer.circuit_size() && head[1] == composer.num_variables() && head[2] == 3,
                "export header: rows, variables, calls (fresh + add_input + range_check)");
     }
