@@ -22,6 +22,8 @@ pub struct pg_ctx {
 }
 pub type pg_col = u64;
 
+pub const PG_FORM_EVALUATIONS: c_int = 0;
+pub const PG_FORM_COEFFICIENTS: c_int = 1;
 pub const PG_OK: c_int = 0;
 pub const PG_ERR_NON_EXISTING_INVERSE: c_int = 1;
 pub const PG_ERR_CUDA: c_int = -1;
@@ -149,6 +151,12 @@ extern "C" {
     pub fn pg_permutation(ctx: *mut pg_ctx, row0: u64, cnt: u64, sigma: *mut u64, dst_on_device: c_int) -> c_int;
     pub fn pg_fft(ctx: *mut pg_ctx, log_n: u32, inverse: c_int, src: *const pg_fr, dst: *mut pg_fr, on_device: c_int) -> c_int;
     pub fn pg_wire_polynomials(ctx: *mut pg_ctx, log_n: u32, dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
+    pub fn pg_sigma_polynomials(ctx: *mut pg_ctx, log_n: u32, form: c_int, dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
+    pub fn pg_permutation_z(ctx: *mut pg_ctx, log_n: u32, beta: *const pg_fr, gamma: *const pg_fr, form: c_int, dst: *mut pg_fr,
+                            dst_on_device: c_int, closing: *mut pg_fr) -> c_int;
+    pub fn pg_permutation_z_rows(ctx: *mut pg_ctx, log_n: u32, n: u64, w_val: *const pg_fr, sigma: *const u64, on_device: c_int,
+                                 beta: *const pg_fr, gamma: *const pg_fr, form: c_int, dst: *mut pg_fr, dst_on_device: c_int,
+                                 closing: *mut pg_fr) -> c_int;
     pub fn pg_msm(ctx: *mut pg_ctx, n: u64, points: *const pg_g1_affine, scalars: *const pg_fr, out: *mut pg_g1_affine, on_device: c_int) -> c_int;
     pub fn pg_srs_powers(ctx: *mut pg_ctx, beta: *const pg_fr, base: *const pg_g1_affine, n: u64, out: *mut pg_g1_affine, out_on_device: c_int) -> c_int;
     pub fn pg_g1_fixed_base_mul(ctx: *mut pg_ctx, n: u64, base: *const pg_g1_affine, scalars: *const pg_fr, out: *mut pg_g1_affine,

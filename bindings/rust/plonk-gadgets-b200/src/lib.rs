@@ -188,6 +188,28 @@ impl BatchComposer {
         self.ok(unsafe { sys::pg_wire_polynomials(self.ctx, log_n, flat.as_mut_ptr() as *mut sys::pg_fr, 0) })?;
         Ok(flat.chunks(n).map(|c| c.to_vec()).collect())
     }
+    /// Preprocessing's sigma polynomials (`compute_permutation_lagrange`, or with `coefficients` `compute_sigma_polynomials`) of
+    /// the composer's rows over the domain 2^log_n: four vectors of 2^log_n scalars.
+    pub fn sigma_polynomials(&mut self, log_n: u32, coefficients: bool) -> Result<Vec<Vec<BlsScalar>>, EngineError> {
+        let n = 1usize << log_n;
+        let form = if coefficients { sys::PG_FORM_COEFFICIENTS } else { sys::PG_FORM_EVALUATIONS };
+        let mut flat = vec![BlsScalar::zero(); 4 * n];
+        self.ok(unsafe { sys::pg_sigma_polynomials(self.ctx, log_n, form, flat.as_mut_ptr() as *mut sys::pg_fr, 0) })?;
+        Ok(flat.chunks(n).map(|c| c.to_vec()).collect())
+    }
+    /// Prover round 2: the grand-product polynomial z over the domain 2^log_n (`compute_fast_permutation_poly`, or with
+    /// `coefficients` `compute_permutation_poly`) for the transcript's beta and gamma, and the product of all 2^log_n ratios
+    /// (one on every composer this API builds).
+    pub fn permutation_z(&mut self, log_n: u32, beta: &BlsScalar, gamma: &BlsScalar, coefficients: bool) -> Result<(Vec<BlsScalar>, BlsScalar), EngineError> {
+        let form = if coefficients { sys::PG_FORM_COEFFICIENTS } else { sys::PG_FORM_EVALUATIONS };
+        let mut z = vec![BlsScalar::zero(); 1usize << log_n];
+        let mut closing = BlsScalar::zero();
+        self.ok(unsafe {
+            sys::pg_permutation_z(self.ctx, log_n, beta as *const BlsScalar as *const sys::pg_fr, gamma as *const BlsScalar as *const sys::pg_fr, form,
+                                  z.as_mut_ptr() as *mut sys::pg_fr, 0, &mut closing as *mut BlsScalar as *mut sys::pg_fr)
+        })?;
+        Ok((z, closing))
+    }
     /// Prover round 1, second half: `commit_key.commit(&w_l_poly)` .. `w_4`.  `powers_of_g` are the CommitKey's G1Affine
     /// powers in the layout of `sys::pg_g1_affine` (x, y Montgomery limbs; all-zero = infinity).
     pub fn commit_wire_polynomials(&mut self, log_n: u32, powers_of_g: &[sys::pg_g1_affine]) -> Result<[sys::pg_g1_affine; 4], EngineError> {

@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define PG_B200_ABI_VERSION 3
+#define PG_B200_ABI_VERSION 4
 
 /* BlsScalar: ref:src/allocated_scalar.rs:9-12 (dusk_plonk::bls12_381::BlsScalar) */
 typedef struct pg_fr { uint64_t l[4]; } pg_fr;
@@ -310,6 +310,32 @@ int pg_export_composer(pg_ctx *ctx, const char *path, uint64_t chunk_rows, uint3
 int pg_fft(pg_ctx *ctx, uint32_t log_n, int inverse, const pg_fr *src, pg_fr *dst, int on_device);
 int pg_wire_polynomials(pg_ctx *ctx, uint32_t log_n, pg_fr *dst, int dst_on_device);
 
+/* ---- permutation argument (SURVEY.md section 8f item 2, continued) ----------------------------------------------------------
+ * Preprocessing's sigma polynomials and round 2 of Prover::prove [DEP dusk-plonk 0.8 src/permutation/permutation.rs, recalled
+ * like the rest of [DEP]].  Domain H = <w> of size N = 2^log_n as in pg_fft; rows n_rows .. N are padding (wire value 0, every
+ * position a fixed point of sigma: pad() pushes zero-variable wires without touching the variable map -- recalled, unpinned).
+ * Coset constants k = (1, K1, K2, K3) = (1, 7, 13, 17) for w_l, w_r, w_o, w_4 (permutation/constants.rs, recalled); the identity of
+ * wire position (i, w) is k_w * w^i.
+ * pg_sigma_polynomials: sigma_w(w^i) = k_{w'} * w^{r'}, r'*4 + w' = pg_permutation's successor of (i, w)
+ *   (compute_permutation_lagrange); PG_FORM_COEFFICIENTS: domain.ifft of that (compute_sigma_polynomials).  dst: 4 x N, column-major.
+ * pg_permutation_z: with wire values v_w(i) and the caller's beta, gamma (host pointers; the transcript is not built):
+ *     num_i = prod_w (v_w(i) + beta*k_w*w^i + gamma),  den_i = prod_w (v_w(i) + beta*sigma_w(w^i) + gamma)
+ *     z_0 = 1,  z_{i+1} = z_i * num_i / den_i                      (compute_fast_permutation_poly; coefficients: compute_permutation_poly)
+ *   dst: N scalars.  *closing (host, may be NULL) = prod_{i<N} num_i / den_i, the element the reference drops: 1 on every composer
+ *   this API builds, for any beta and gamma.  A zero den_i (the reference panics in invert().unwrap(), e.g. beta = gamma = 0 on a row
+ *   with the zero variable) is PG_ERR_ARG and pg_last_error names the first such row.
+ * Both: PG_ERR_ARG when 2^log_n < the circuit size or log_n > 32, or beta / gamma is not fully reduced; PG_ERR_STATE on a ctx with a
+ *   communicator of more than one rank (a sharded z needs the other ranks' carries: not built).  They synchronise the ctx stream.
+ * pg_permutation_z_rows: the same over caller-supplied rows (the pg_check_rows counterpart): w_val 4 x n wire values, sigma 4 x n
+ *   positions in pg_permutation's encoding (row*4 + wire), column-major, both host or both device memory; rows n .. N are padding.
+ *   A sigma entry >= 4*N or an unreduced wire value is counted on the device and reported as PG_ERR_ARG by this call. */
+enum { PG_FORM_EVALUATIONS = 0, PG_FORM_COEFFICIENTS = 1 };
+int pg_sigma_polynomials(pg_ctx *ctx, uint32_t log_n, int form, pg_fr *dst, int dst_on_device);
+int pg_permutation_z(pg_ctx *ctx, uint32_t log_n, const pg_fr *beta, const pg_fr *gamma, int form, pg_fr *dst, int dst_on_device,
+                     pg_fr *closing);
+int pg_permutation_z_rows(pg_ctx *ctx, uint32_t log_n, uint64_t n, const pg_fr *w_val, const uint64_t *sigma, int on_device,
+                          const pg_fr *beta, const pg_fr *gamma, int form, pg_fr *dst, int dst_on_device, pg_fr *closing);
+
 /* ---- commitments (SURVEY.md section 8f item 2, second half) -----------------------------------------------------------------
  * KZG commitments of coefficient vectors in the BLS12-381 group G1 [DEP dusk-plonk 0.8 CommitKey::commit =
  * dusk-bls12_381 msm_variable_base(&powers_of_g, &poly.coeffs); Prover::prove computes w_l_poly_commit .. w_4_poly_commit right
@@ -390,7 +416,8 @@ int pg_measure_imad_peak(pg_ctx *ctx, double *wide_mac_per_s, double *imad_per_s
 int pg_microbench(pg_ctx *ctx, int mode, double *ops_per_s);
 
 /* Element-wise Fr self-test kernels (op: 0 mul, 1 add, 2 sub, 3 neg, 4 invert-or-zero (batch inversion), 5 from_mont,
- * 6 mul via the portable CIOS path).  a, b, out: host arrays of n scalars. */
+ * 6 mul via the portable CIOS path, 7 exclusive prefix product out[0] = 1, out[i] = a[0]*..*a[i-1] (the grand-product scan of
+ * pg_permutation_z)).  a, b, out: host arrays of n scalars. */
 int pg_fr_op(pg_ctx *ctx, int op, uint64_t n, const pg_fr *a, const pg_fr *b, pg_fr *out);
 
 #ifdef __cplusplus

@@ -46,7 +46,7 @@ class pg_check_stats(C.Structure):
     _fields_ = [("launches", C.c_uint64 * 8), ("rows", C.c_uint64 * 8)]
 
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # every symbol include/pg_b200.h declares: name -> (restype, argtypes)
 _vp, _u64, _i32, _u32 = C.c_void_p, C.c_uint64, C.c_int, C.c_uint32
@@ -92,6 +92,9 @@ SIGNATURES = {
     "pg_export_composer": (_i32, [_vp, C.c_char_p, _u64, _u32]),
     "pg_fft": (_i32, [_vp, _u32, _i32, _vp, _vp, _i32]),
     "pg_wire_polynomials": (_i32, [_vp, _u32, _vp, _i32]),
+    "pg_sigma_polynomials": (_i32, [_vp, _u32, _i32, _vp, _i32]),
+    "pg_permutation_z": (_i32, [_vp, _u32, _vp, _vp, _i32, _vp, _i32, _vp]),
+    "pg_permutation_z_rows": (_i32, [_vp, _u32, _u64, _vp, _vp, _i32, _vp, _vp, _i32, _vp, _i32, _vp]),
     "pg_msm": (_i32, [_vp, _u64, _vp, _vp, _vp, _i32]),
     "pg_srs_powers": (_i32, [_vp, _vp, _vp, _u64, _vp, _i32]),
     "pg_g1_fixed_base_mul": (_i32, [_vp, _u64, _vp, _vp, _vp, _i32]),

@@ -29,6 +29,7 @@ from . import _lib
 CHECK_GENERIC, CHECK_SPARSE = 0, 1
 F_TIMING = 1
 F_FUSED_CHECK = 2
+FORM_EVALUATIONS, FORM_COEFFICIENTS = 0, 1
 UINT64_MAX = 2 ** 64 - 1
 
 
@@ -398,6 +399,54 @@ class StandardComposer:
         dst = np.empty((4, 1 << log_n, 4), dtype=np.uint64)
         self._ok(self._L.pg_wire_polynomials(self._ctx, log_n, dst.ctypes.data_as(C.c_void_p), 0), "pg_wire_polynomials")
         return dst
+
+    # -- permutation argument: preprocessing's sigma polynomials and prover round 2's z(X) ([DEP] dusk-plonk 0.8 permutation.rs)
+    def _domain(self, log_n):
+        log_n = self.domain_log_size() if log_n is None else log_n
+        if not 0 <= log_n <= 32:
+            raise EngineError(-2, "permutation argument", f"log_n = {log_n} is outside 0..32")
+        return log_n
+
+    def sigma_polynomials(self, log_n: int | None = None, form: int = FORM_EVALUATIONS, out=None):
+        """sigma_w over the domain 2^log_n: (4, 2^log_n, 4) uint64 evaluations or coefficients (host array, or written to the
+        device tensor `out`)."""
+        log_n = self._domain(log_n)
+        if out is not None:
+            self._ok(self._L.pg_sigma_polynomials(self._ctx, log_n, form, C.c_void_p(out.data_ptr()), 1), "pg_sigma_polynomials")
+            return out
+        dst = np.empty((4, 1 << log_n, 4), dtype=np.uint64)
+        self._ok(self._L.pg_sigma_polynomials(self._ctx, log_n, form, dst.ctypes.data_as(C.c_void_p), 0), "pg_sigma_polynomials")
+        return dst
+
+    def _z_call(self, fn, what, log_n, head, beta, gamma, form, out):
+        b = np.ascontiguousarray(beta, dtype=np.uint64).reshape(4); g = np.ascontiguousarray(gamma, dtype=np.uint64).reshape(4)
+        closing = np.zeros(4, dtype=np.uint64)
+        vp = lambda x: x.ctypes.data_as(C.c_void_p)
+        if out is not None:
+            self._ok(fn(self._ctx, log_n, *head, vp(b), vp(g), form, C.c_void_p(out.data_ptr()), 1, vp(closing)), what)
+            return out, closing
+        dst = np.empty((1 << log_n, 4), dtype=np.uint64)
+        self._ok(fn(self._ctx, log_n, *head, vp(b), vp(g), form, vp(dst), 0, vp(closing)), what)
+        return dst, closing
+
+    def permutation_z(self, beta, gamma, log_n: int | None = None, form: int = FORM_EVALUATIONS, out=None):
+        """(z, closing): the grand-product polynomial over the domain 2^log_n ((2^log_n, 4) uint64, or the device tensor `out`)
+        and the product of all 2^log_n ratios ((4,) uint64; one on every honestly wired composer)."""
+        return self._z_call(self._L.pg_permutation_z, "pg_permutation_z", self._domain(log_n), (), beta, gamma, form, out)
+
+    def permutation_z_rows(self, w_val, sigma, beta, gamma, log_n: int, form: int = FORM_EVALUATIONS, out=None):
+        """permutation_z over caller-supplied rows: w_val (4, n, 4) wire values and sigma (4, n) positions (row*4 + wire), both host
+        arrays or both device tensors; rows n .. 2^log_n are padding."""
+        if hasattr(w_val, "data_ptr"):
+            n = w_val.shape[1]
+            head = (n, C.c_void_p(w_val.data_ptr()), C.c_void_p(sigma.data_ptr()), 1)
+        else:
+            w = np.ascontiguousarray(w_val, dtype=np.uint64); s = np.ascontiguousarray(sigma, dtype=np.uint64)
+            n = w.shape[1]
+            if s.shape != (4, n):
+                raise ValueError("permutation_z_rows: sigma must be (4, n) for w_val (4, n, 4)")
+            head = (n, w.ctypes.data_as(C.c_void_p), s.ctypes.data_as(C.c_void_p), 0)
+        return self._z_call(self._L.pg_permutation_z_rows, "pg_permutation_z_rows", log_n, head, beta, gamma, form, out)
 
     # -- commitments: G1 multi-scalar multiplication, SRS powers, wire-polynomial commitments ([DEP] dusk-plonk 0.8 / dusk-bls12_381)
     @staticmethod

@@ -14,6 +14,7 @@
 //   SelectZeroBody  /root/reference/src/scalar.rs:21-27        SelectOneBody  /root/reference/src/scalar.rs:36-59
 #pragma once
 #include "layout.h"
+#include "ntt.cuh"
 
 namespace pg {
 
@@ -974,6 +975,56 @@ struct PermBody {
             a.sigma[(uint64_t)w * a.n + tix] = out;
         }
     }
+};
+
+// ---------------------------------------------------------------------------------------------------- permutation argument
+// [DEP] dusk-plonk 0.8 permutation.rs.  The identity of wire position (i, w) is k_w * w^i, k = (1, K1, K2, K3); sigma maps it
+// to the identity of its cycle successor.  Positions: PermBody's encoding row*4 + wire; rows >= n_sig (padding) map to themselves.
+PG_HD uint64_t perm_successor(const unsigned long long* sigma, uint64_t n_sig, uint64_t i, uint32_t w) {
+    return i < n_sig ? sigma[(uint64_t)w * n_sig + i] : i * 4ull + w;
+}
+// sigma_w(w^i) = k_{w'} * w^{r'} (compute_permutation_lagrange): out is 4 columns of n evaluations
+struct PermSigmaBody {
+    struct Args { const unsigned long long* sigma; uint64_t n_sig; uint64_t n; const uint4* tw; uint32_t log_n; Fr k[4]; uint4* out; };
+    PG_HD static void run(const Args& a, uint64_t i) {
+#pragma unroll
+        for (uint32_t w = 0; w < 4; w++) {
+            const uint64_t p = perm_successor(a.sigma, a.n_sig, i, w);
+            aos_store(a.out, (uint64_t)w * a.n + i, fr_mul(a.k[p & 3u], domain_pow(a.tw, a.log_n, p >> 2)));
+        }
+    }
+};
+// The ratios of the grand product (compute_fast_permutation_poly), inside k_batch_inv's two walks (in_slot 0 = den, out_slot 1):
+//   num_i = prod_w (v_w(i) + beta*k_w*w^i + gamma),  den_i = prod_w (v_w(i) + beta*sigma_w(w^i) + gamma)
+// pre parks num_i in `ratio` and hands den_i to the inversion; post writes ratio_i = num_i * den_i^-1.  A zero den_i (the reference
+// panics in invert().unwrap()) is counted in CNT_N_ERR / CNT_FIRST_ERR -- the zero-aware inversion would store 0 silently.
+// check (caller-supplied rows): a sigma entry >= 4n or an unreduced wire value is counted in CNT_UNSAT / CNT_FIRST_BAD (and the
+// position is read as a fixed point, so no access leaves the twiddle table).
+struct PermRatioHook {
+    struct Args { const uint4* w; uint64_t n; const unsigned long long* sigma; uint64_t n_sig; const uint4* tw; uint32_t log_n;
+                  Fr bk[4]; Fr gamma; uint4* den; uint4* ratio; unsigned long long* counters; int check; };
+    PG_HD static Fr pre(const Args& a, uint64_t i) {
+        const Fr wi = domain_pow(a.tw, a.log_n, i);
+        Fr num = fr_one(), den = fr_one();
+        bool bad = false;
+#pragma unroll
+        for (uint32_t w = 0; w < 4; w++) {
+            const Fr v = aos_load(a.w, (uint64_t)w * a.n + i);
+            uint64_t p = perm_successor(a.sigma, a.n_sig, i, w);
+            if (a.check) {
+                if (!fr_is_reduced(v)) bad = true;
+                if (p >= 4ull * a.n) { bad = true; p = i * 4ull + w; }
+            }
+            num = fr_mul(num, fr_add(fr_add(v, fr_mul(a.bk[w], wi)), a.gamma));
+            den = fr_mul(den, fr_add(fr_add(v, fr_mul(a.bk[p & 3u], domain_pow(a.tw, a.log_n, p >> 2))), a.gamma));
+        }
+        if (bad) { counter_add(a.counters + CNT_UNSAT, 1ull); counter_min(a.counters + CNT_FIRST_BAD, (unsigned long long)i); }
+        if (fr_is_zero(den)) { counter_add(a.counters + CNT_N_ERR, 1ull); counter_min(a.counters + CNT_FIRST_ERR, (unsigned long long)i); }
+        aos_store(a.ratio, i, num);
+        tab_store_fr(a.den, a.n, 0, i, den);
+        return den;
+    }
+    PG_HD static void post(const Args& a, uint64_t i, const Fr&, const Fr& den_inv) { aos_store(a.ratio, i, fr_mul(aos_load(a.ratio, i), den_inv)); }
 };
 
 // ---------------------------------------------------------------------------------------------------- synthetic inputs

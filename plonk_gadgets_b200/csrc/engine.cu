@@ -425,6 +425,26 @@ public:
         toc();
         return launched("k_ntt_pass");
     }
+    // exclusive prefix product (scan.cuh) of n scalars; *total = product of all; scratch: fr_scan_scratch(n) scalars
+    bool run_fr_scan(const uint4* in, uint4* out, uint64_t n, uint4* total, uint4* scratch) {
+        if (!n) return true;
+        tic(CLS_OTHER, 0);
+        const bool ok = fr_scan_level(in, out, n, total, scratch);
+        toc();
+        return ok;
+    }
+    bool fr_scan_level(const uint4* in, uint4* out, uint64_t n, uint4* total, uint4* scratch) {
+        if (n <= SCAN_TILE) {
+            k_fr_scan_apply<<<1, SCAN_THREADS, 0, stream>>>(in, out, n, nullptr, total);
+            return launched("k_fr_scan_apply");
+        }
+        const uint64_t tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
+        k_fr_scan_reduce<<<(unsigned)tiles, SCAN_THREADS, 0, stream>>>(in, n, scratch);
+        if (!launched("k_fr_scan_reduce")) return false;
+        if (!fr_scan_level(scratch, scratch, tiles, total, scratch + 2 * tiles)) return false;      // tile totals -> their exclusive prefixes
+        k_fr_scan_apply<<<(unsigned)tiles, SCAN_THREADS, 0, stream>>>(in, out, n, scratch, nullptr);
+        return launched("k_fr_scan_apply");
+    }
     bool run_check_rows(const CheckRowsBody::Args& a) {
         tic(CLS_CHECK, a.n);
         k_check_rows<<<grid_for(a.n), BLOCK, 0, stream>>>(a);
@@ -504,6 +524,8 @@ public:
     }
     bool imad_peak(double* wide, double* lo) { return ubench(UB_WIDE_ACC, wide) && ubench(UB_IMAD_LO, lo); }
 };
+
+static_assert(has_fr_scan<CudaBackend>::value, "the shipped library computes the grand product with the device-wide scan of scan.cuh");
 
 }  // namespace pg
 

@@ -18,6 +18,8 @@
 //   bool run_msm_buckets(const MsmBucketBody::Args&)             -- one thread per part of a bucket run (launch shape chosen by the backend)
 //   bool exclusive_sum(const uint32_t* in, uint32_t* out, uint64_t n)
 //   bool run_ntt_pass(const NttPassArgs&, uint64_t n_blocks)    -- one group of butterfly stages over all tiles (ntt.cuh)
+//   bool run_fr_scan(const uint4* in, uint4* out, uint64_t n, uint4* total, uint4* scratch) -- exclusive prefix product (scan.cuh);
+//        optional: a backend without it (the test-only loop backend) runs FrScanSerialBody, the defining serial loop
 //   bool upload_pow2(const Fr*), bool imad_peak(double*, double*), bool ubench(int, double*), timing(pg_timing*, bool reset)
 #pragma once
 #include <stdio.h>
@@ -26,10 +28,12 @@
 #include <map>
 #include <string>
 #include <vector>
+#include <type_traits>
 #include "../../include/pg_b200.h"
 #include "templates.hpp"
 #include "shard.hpp"
 #include "ntt.cuh"
+#include "scan.cuh"
 #include "msm.cuh"
 
 namespace pg {
@@ -83,6 +87,10 @@ inline Fr fr_from_pg(const pg_fr& x) {
     for (int i = 0; i < 4; i++) { r.v[2 * i] = (uint32_t)x.l[i]; r.v[2 * i + 1] = (uint32_t)(x.l[i] >> 32); }
     return r;
 }
+
+// whether a backend brings its own device-wide prefix product (Engine::fr_scan)
+template <class B, class = void> struct has_fr_scan : std::false_type {};
+template <class B> struct has_fr_scan<B, std::void_t<decltype(&B::run_fr_scan)>> : std::true_type {};
 
 template <class BE>
 class Engine {
@@ -1154,6 +1162,16 @@ public:
         release_scratch_from(mark);
         return rc;
     }
+    // to_scalars(w_l..w_4) of the composer's rows, padded with zeros up to the domain size n: 4 columns of n scalars in buf
+    int wire_values(uint64_t n, uint4* buf) {
+        int rc = materialize_dev(0, n_rows, n, nullptr, buf, nullptr, nullptr);
+        if (rc) return rc;
+        for (int w = 0; w < 4 && n > n_rows; w++) {
+            NttZeroBody::Args z{buf + 2 * (uint64_t)w * n, n_rows, n - n_rows};
+            if (!be.template run_simple<NttZeroBody>(z, z.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "padding kernel");
+        }
+        return PG_OK;
+    }
     // dst: 4 columns (w_l, w_r, w_o, w_4) of 2^log_n coefficients each
     int wire_polynomials(uint32_t log_n, pg_fr* dst, int dst_on_device) {
         if (log_n > NTT_TWO_ADICITY || (1ull << log_n) < n_rows || !dst) return fail(PG_ERR_ARG, "wire_polynomials: domain smaller than the circuit, larger than 2^32, or null buffer");
@@ -1161,16 +1179,10 @@ public:
         const size_t mark = scratch.size();
         uint4* buf = reinterpret_cast<uint4*>(dst);
         if (!dst_on_device) { buf = (uint4*)dalloc(bytes); if (!buf) return fail(PG_ERR_OOM, "wire polynomial buffer"); scratch.push_back(buf); }
-        int rc = materialize_dev(0, n_rows, n, nullptr, buf, nullptr, nullptr);      // to_scalars(w_l..w_4)
+        int rc = wire_values(n, buf);
         if (rc) return rc;
-        for (int w = 0; w < 4; w++) {
-            uint4* col = buf + 2 * (uint64_t)w * n;
-            if (n > n_rows) {                                                        // pad with zeros up to the domain size
-                NttZeroBody::Args z{col, n_rows, n - n_rows};
-                if (!be.template run_simple<NttZeroBody>(z, z.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "padding kernel");
-            }
-            if ((rc = ntt_inplace(col, log_n, true))) return rc;                     // domain.ifft
-        }
+        for (int w = 0; w < 4; w++)
+            if ((rc = ntt_inplace(buf + 2 * (uint64_t)w * n, log_n, true))) return rc;   // domain.ifft
         if (dst_on_device) return PG_OK;
         rc = deliver(dst, buf, bytes, 0);
         release_scratch_from(mark);
@@ -1266,6 +1278,141 @@ public:
         const int rc = deliver(sigma, out, 4 * cnt * sizeof(uint64_t), 0);
         release_scratch_from(mark);
         return rc;
+    }
+
+    // ------------------------------------------------------------------------------------------------ permutation argument
+    // Preprocessing's sigma polynomials and prover round 2's z(X) [DEP dusk-plonk 0.8 permutation.rs]; bodies.cuh PermSigmaBody /
+    // PermRatioHook, scan.cuh.  Coset constants k = (1, K1, K2, K3) = (1, 7, 13, 17) (permutation/constants.rs, recalled).
+    static Fr perm_coset(uint32_t w) { static const uint32_t k[4] = {1, 7, 13, 17}; Fr raw = fr_zero(); raw.v[0] = k[w]; return fr_to_mont(raw); }
+    int perm_domain(const char* who, uint32_t log_n, uint64_t rows, int form) {
+        if (log_n > NTT_TWO_ADICITY || (1ull << log_n) < rows) return fail(PG_ERR_ARG, std::string(who) + ": domain smaller than the circuit or larger than 2^32");
+        if (form != PG_FORM_EVALUATIONS && form != PG_FORM_COEFFICIENTS) return fail(PG_ERR_ARG, std::string(who) + ": form must be PG_FORM_EVALUATIONS or PG_FORM_COEFFICIENTS");
+        return PG_OK;
+    }
+    // a sharded composer holds one rank's rows: the grand product would need the other ranks' carries (not built)
+    int perm_unsharded(const char* who) {
+        return be.comm_world() > 1 ? fail(PG_ERR_STATE, std::string(who) + ": the composer is sharded over a communicator; a sharded permutation argument is not built") : PG_OK;
+    }
+    // the composer's copy-constraint map (rows 0 .. n_rows) on the device, parked in `scratch`
+    unsigned long long* perm_map_dev(int* rc) {
+        unsigned long long* d = (unsigned long long*)dalloc(4 * (n_rows ? n_rows : 1) * sizeof(uint64_t));
+        if (!d) { *rc = fail(PG_ERR_OOM, "permutation buffer"); return nullptr; }
+        scratch.push_back(d);
+        *rc = permutation(0, n_rows, reinterpret_cast<uint64_t*>(d), 1);
+        return *rc ? nullptr : d;
+    }
+    int sigma_polynomials(uint32_t log_n, int form, pg_fr* dst, int dst_on_device) {
+        int rc;
+        if ((rc = perm_unsharded("sigma_polynomials")) || (rc = perm_domain("sigma_polynomials", log_n, n_rows, form))) return rc;
+        if (!dst) return fail(PG_ERR_ARG, "sigma_polynomials: null buffer");
+        const uint64_t n = 1ull << log_n; const size_t bytes = 4 * n * sizeof(pg_fr);
+        const size_t mark = scratch.size();
+        uint4* buf = reinterpret_cast<uint4*>(dst);
+        if (!dst_on_device) { buf = (uint4*)dalloc(bytes); if (!buf) return fail(PG_ERR_OOM, "sigma buffer"); scratch.push_back(buf); }
+        const unsigned long long* sig = perm_map_dev(&rc); if (!sig) return rc;
+        if (log_n && (rc = ntt_twiddles(log_n))) return rc;
+        PermSigmaBody::Args a; memset(&a, 0, sizeof(a));
+        a.sigma = sig; a.n_sig = n_rows; a.n = n; a.tw = log_n ? ntt_tw : nullptr; a.log_n = log_n; a.out = buf;
+        for (uint32_t w = 0; w < 4; w++) a.k[w] = perm_coset(w);
+        if (!be.template run_simple<PermSigmaBody>(a, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "sigma kernel");   // compute_permutation_lagrange
+        for (int w = 0; w < 4 && form == PG_FORM_COEFFICIENTS; w++)
+            if ((rc = ntt_inplace(buf + 2 * (uint64_t)w * n, log_n, true))) return rc;      // compute_sigma_polynomials: domain.ifft
+        if (!dst_on_device) { if ((rc = deliver(dst, buf, bytes, 0))) return rc; }
+        else if (!be.sync()) return fail(PG_ERR_CUDA, "sync");                            // the map's tables go back to the pool
+        release_scratch_from(mark);
+        return PG_OK;
+    }
+    int permutation_z(uint32_t log_n, const pg_fr* beta, const pg_fr* gamma, int form, pg_fr* dst, int dst_on_device, pg_fr* closing) {
+        int rc;
+        if ((rc = perm_unsharded("permutation_z")) || (rc = perm_domain("permutation_z", log_n, n_rows, form))) return rc;
+        if ((rc = perm_scalars("permutation_z", beta, gamma, dst))) return rc;
+        const uint64_t n = 1ull << log_n;
+        const size_t mark = scratch.size();
+        uint4* w = (uint4*)dalloc(4 * n * sizeof(pg_fr)); if (!w) return fail(PG_ERR_OOM, "wire value buffer");
+        scratch.push_back(w);
+        if ((rc = wire_values(n, w))) return rc;
+        const unsigned long long* sig = perm_map_dev(&rc); if (!sig) return rc;
+        return permutation_z_dev(log_n, w, sig, n_rows, false, beta, gamma, form, dst, dst_on_device, closing, mark);
+    }
+    // the same over caller-supplied rows: w_val 4 x n_in, sigma 4 x n_in (row*4 + wire), rows n_in .. 2^log_n padding
+    int permutation_z_rows(uint32_t log_n, uint64_t n_in, const pg_fr* w_val, const uint64_t* sigma, int on_device, const pg_fr* beta,
+                           const pg_fr* gamma, int form, pg_fr* dst, int dst_on_device, pg_fr* closing) {
+        int rc;
+        if ((rc = perm_domain("permutation_z_rows", log_n, n_in, form))) return rc;
+        if ((rc = perm_scalars("permutation_z_rows", beta, gamma, dst))) return rc;
+        if (n_in && (!w_val || !sigma)) return fail(PG_ERR_ARG, "permutation_z_rows: null rows");
+        const uint64_t n = 1ull << log_n;
+        const size_t mark = scratch.size();
+        uint4* w = (uint4*)dalloc(4 * n * sizeof(pg_fr)); if (!w) return fail(PG_ERR_OOM, "wire value buffer");
+        scratch.push_back(w);
+        for (uint64_t c = 0; c < 4; c++) {                                                  // stride n_in -> stride n, zero padding
+            uint4* col = w + 2 * c * n;
+            if (n_in && !(on_device ? be.d2d(col, w_val + c * n_in, n_in * sizeof(pg_fr)) : be.h2d(col, w_val + c * n_in, n_in * sizeof(pg_fr))))
+                return fail(PG_ERR_CUDA, "row copy");
+            NttZeroBody::Args z{col, n_in, n - n_in};
+            if (n > n_in && !be.template run_simple<NttZeroBody>(z, z.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "padding kernel");
+        }
+        const unsigned long long* sig = reinterpret_cast<const unsigned long long*>(sigma);
+        if (!on_device && n_in) {
+            void* d = dalloc(4 * n_in * sizeof(uint64_t)); if (!d) return fail(PG_ERR_OOM, "sigma staging buffer");
+            scratch.push_back(d);
+            if (!be.h2d(d, sigma, 4 * n_in * sizeof(uint64_t))) return fail(PG_ERR_CUDA, "sigma copy");
+            sig = (const unsigned long long*)d;
+        }
+        return permutation_z_dev(log_n, w, sig, n_in, true, beta, gamma, form, dst, dst_on_device, closing, mark);
+    }
+    int perm_scalars(const char* who, const pg_fr* beta, const pg_fr* gamma, const pg_fr* dst) {
+        if (!beta || !gamma || !dst) return fail(PG_ERR_ARG, std::string(who) + ": null argument");
+        if (!host_reduced(*beta) || !host_reduced(*gamma)) return fail(PG_ERR_ARG, std::string(who) + ": beta / gamma not fully reduced (>= q)");
+        return PG_OK;
+    }
+    // exclusive prefix product of n scalars, *total = their product: the backend's device-wide scan (CudaBackend::run_fr_scan, scan.cuh;
+    // engine.cu asserts that it has one), else FrScanSerialBody as one unit of work
+    bool fr_scan(const uint4* in, uint4* out, uint64_t n, uint4* total, uint4* scratch) {
+        if constexpr (has_fr_scan<BE>::value) return be.run_fr_scan(in, out, n, total, scratch);
+        else { (void)scratch; const FrScanSerialBody::Args a{in, out, n, total}; return be.template run_simple<FrScanSerialBody>(a, 1, CLS_OTHER); }
+    }
+    // ratios fused into the batch inversion (k_batch_inv<PermRatioHook>), exclusive prefix product (z and the closing product),
+    // optionally domain.ifft; synchronises to read the zero-denominator / bad-row counters
+    int permutation_z_dev(uint32_t log_n, const uint4* w, const unsigned long long* sig, uint64_t n_sig, bool check_rows, const pg_fr* beta,
+                          const pg_fr* gamma, int form, pg_fr* dst, int dst_on_device, pg_fr* closing, size_t mark) {
+        const uint64_t n = 1ull << log_n;
+        int rc;
+        uint4* z = reinterpret_cast<uint4*>(dst);
+        if (!dst_on_device) { z = (uint4*)dalloc(n * sizeof(pg_fr)); if (!z) return fail(PG_ERR_OOM, "z buffer"); scratch.push_back(z); }
+        uint4* tab = (uint4*)dalloc(2 * n * sizeof(pg_fr)); if (!tab) return fail(PG_ERR_OOM, "inversion table");
+        scratch.push_back(tab);
+        uint4* tot = (uint4*)dalloc((1 + fr_scan_scratch(n)) * sizeof(pg_fr)); if (!tot) return fail(PG_ERR_OOM, "scan scratch");
+        scratch.push_back(tot);
+        if (log_n && (rc = ntt_twiddles(log_n))) return rc;
+        if ((rc = reset_counters())) return rc;
+        const Fr b = fr_from_pg(*beta);
+        PermRatioHook::Args h; memset(&h, 0, sizeof(h));
+        h.w = w; h.n = n; h.sigma = sig; h.n_sig = n_sig; h.tw = log_n ? ntt_tw : nullptr; h.log_n = log_n;
+        for (uint32_t k = 0; k < 4; k++) h.bk[k] = fr_mul(b, perm_coset(k));
+        h.gamma = fr_from_pg(*gamma); h.den = tab; h.ratio = z; h.counters = d_counters; h.check = check_rows ? 1 : 0;
+        BatchInvArgs inv; memset(&inv, 0, sizeof(inv));
+        inv.fr = tab; inv.stride = n; inv.n = n; inv.n_pairs = 1; inv.in_slot[0] = 0; inv.out_slot[0] = 1;
+        if (!be.template run_batch_inv_fused<PermRatioHook>(inv, h, CLS_OTHER)) return fail(PG_ERR_CUDA, "permutation ratio kernel");
+        if (!fr_scan(z, z, n, tot, tot + 2)) return fail(PG_ERR_CUDA, "grand-product scan");
+        if (form == PG_FORM_COEFFICIENTS && (rc = ntt_inplace(z, log_n, true))) return rc;      // compute_permutation_poly: domain.ifft(z)
+        unsigned long long c[CNT_WORDS];
+        if ((rc = read_counters(c))) return rc;
+        if (c[CNT_UNSAT]) {
+            char msg[200];
+            snprintf(msg, sizeof(msg), "permutation_z_rows: %llu row(s) with a sigma entry >= 4 * 2^%u or an unreduced wire value, first at row %llu",
+                     c[CNT_UNSAT], log_n, c[CNT_FIRST_BAD]);
+            return fail(PG_ERR_ARG, msg);
+        }
+        if (c[CNT_N_ERR]) {
+            char msg[200];
+            snprintf(msg, sizeof(msg), "permutation_z: %llu zero denominator(s) v + beta*sigma + gamma, first at row %llu", c[CNT_N_ERR], c[CNT_FIRST_ERR]);
+            return fail(PG_ERR_ARG, msg);
+        }
+        if (closing && (rc = deliver(closing, tot, sizeof(pg_fr), 0))) return rc;
+        if (!dst_on_device && (rc = deliver(dst, z, n * sizeof(pg_fr), 0))) return rc;
+        release_scratch_from(mark);
+        return PG_OK;
     }
 
     // ------------------------------------------------------------------------------------------------ export (SURVEY.md 8f.1)
@@ -1389,6 +1536,11 @@ public:
             DevTab view; memset(&view, 0, sizeof(view)); view.fr = tab; view.stride = n;
             ColReadBody::Args rd{view, loc_make(LOC_FR, 0, 1), dout, n};
             ok = be.template run_simple<AddInputBody>(in, n, CLS_OTHER) && be.run_batch_inv(inv, CLS_OTHER) && be.template run_simple<ColReadBody>(rd, n, CLS_OTHER);
+        }
+        else if (op == 7) {  // exclusive prefix product through the grand-product scan (scan.cuh)
+            uint4* tot = (uint4*)dalloc((1 + fr_scan_scratch(n)) * sizeof(pg_fr)); if (!tot) return fail(PG_ERR_OOM, "fr_op scan scratch");
+            scratch.push_back(tot);
+            ok = fr_scan(da, dout, n, tot, tot + 2);
         }
         else { FrOpBody::Args g{op, da, db, dout, n}; ok = be.template run_simple<FrOpBody>(g, n, CLS_OTHER); }
         if (!ok) return fail(PG_ERR_CUDA, "fr_op kernel");
@@ -1606,13 +1758,9 @@ public:
         uint4* vals = (uint4*)dalloc(4 * n * sizeof(pg_fr)); if (!vals) return fail(PG_ERR_OOM, "wire value buffer"); scratch.push_back(vals);
         uint4* d_out = (uint4*)dalloc(4 * sizeof(pg_g1_affine)); if (!d_out) return fail(PG_ERR_OOM, "commitments"); scratch.push_back(d_out);
         uint4* win = (uint4*)dalloc(4 * MSM_MAX_WINDOWS * sizeof(G1X)); if (!win) return fail(PG_ERR_OOM, "window sums"); scratch.push_back(win);
-        if ((rc = materialize_dev(0, n_rows, n, nullptr, vals, nullptr, nullptr))) return rc;       // to_scalars(w_l..w_4)
+        if ((rc = wire_values(n, vals))) return rc;
         for (int w = 0; w < 4; w++) {
             uint4* col = vals + 2 * (uint64_t)w * n;
-            if (n > n_rows) {
-                NttZeroBody::Args z{col, n_rows, n - n_rows};
-                if (!be.template run_simple<NttZeroBody>(z, z.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "padding kernel");
-            }
             if ((rc = msm_dev(n, dp, col, nullptr, win + (size_t)w * msm_plan(n).n_windows * (sizeof(G1X) / sizeof(uint4))))) return rc;
         }
         if ((rc = msm_finish(n, win, 4, d_out))) return rc;

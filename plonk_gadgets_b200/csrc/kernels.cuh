@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <type_traits>
 #include "bodies.cuh"
+#include "scan.cuh"
 
 namespace pg {
 

@@ -55,6 +55,13 @@ struct NttTwiddleBody {
     }
 };
 
+// w^j for any j < n from that table: w^(j + n/2) = -w^j.  log_n == 0 (one point, no table): 1.
+PG_HD Fr domain_pow(const uint4* tw, uint32_t log_n, uint64_t j) {
+    if (!log_n) return fr_one();
+    const uint64_t h = 1ull << (log_n - 1u);
+    return j <= h ? aos_load(tw, j) : fr_neg(aos_load(tw, j - h));
+}
+
 // zero-fill of the padding rows [n0, n) of a column
 struct NttZeroBody {
     struct Args { uint4* data; uint64_t n0; uint64_t n; };

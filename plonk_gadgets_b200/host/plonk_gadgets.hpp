@@ -154,6 +154,22 @@ public:
         ok(pg_wire_polynomials(ctx_, log_n, reinterpret_cast<pg_fr*>(out.data()), 0), "pg_wire_polynomials");
         return out;
     }
+    /// preprocessing's sigma polynomials over the domain 2^log_n (evaluations, or coefficients): 4 x 2^log_n scalars
+    std::vector<BlsScalar> sigma_polynomials(uint32_t log_n, bool coefficients = false) {
+        std::vector<BlsScalar> out((size_t)4 << log_n);
+        ok(pg_sigma_polynomials(ctx_, log_n, coefficients ? PG_FORM_COEFFICIENTS : PG_FORM_EVALUATIONS, reinterpret_cast<pg_fr*>(out.data()), 0),
+           "pg_sigma_polynomials");
+        return out;
+    }
+    /// prover round 2: z over the domain 2^log_n for the caller's beta, gamma; *closing = product of all ratios (may be null)
+    std::vector<BlsScalar> permutation_z(uint32_t log_n, const BlsScalar& beta, const BlsScalar& gamma, bool coefficients = false,
+                                         BlsScalar* closing = nullptr) {
+        std::vector<BlsScalar> out((size_t)1 << log_n);
+        ok(pg_permutation_z(ctx_, log_n, reinterpret_cast<const pg_fr*>(&beta), reinterpret_cast<const pg_fr*>(&gamma),
+                            coefficients ? PG_FORM_COEFFICIENTS : PG_FORM_EVALUATIONS, reinterpret_cast<pg_fr*>(out.data()), 0,
+                            reinterpret_cast<pg_fr*>(closing)), "pg_permutation_z");
+        return out;
+    }
     /// EvaluationDomain::fft / ifft of 2^k scalars
     std::vector<BlsScalar> fft(const std::vector<BlsScalar>& v, bool inverse) {
         uint32_t log_n = 0; while ((1ull << log_n) < v.size()) log_n++;
