@@ -157,6 +157,10 @@ extern "C" {
     pub fn pg_permutation_z_rows(ctx: *mut pg_ctx, log_n: u32, n: u64, w_val: *const pg_fr, sigma: *const u64, on_device: c_int,
                                  beta: *const pg_fr, gamma: *const pg_fr, form: c_int, dst: *mut pg_fr, dst_on_device: c_int,
                                  closing: *mut pg_fr) -> c_int;
+    pub fn pg_selector_polynomials(ctx: *mut pg_ctx, log_n: u32, form: c_int, dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
+    pub fn pg_public_input_polynomial(ctx: *mut pg_ctx, log_n: u32, form: c_int, dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
+    pub fn pg_quotient(ctx: *mut pg_ctx, log_n: u32, alpha: *const pg_fr, beta: *const pg_fr, gamma: *const pg_fr, range_challenge: *const pg_fr,
+                       dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
     pub fn pg_msm(ctx: *mut pg_ctx, n: u64, points: *const pg_g1_affine, scalars: *const pg_fr, out: *mut pg_g1_affine, on_device: c_int) -> c_int;
     pub fn pg_srs_powers(ctx: *mut pg_ctx, beta: *const pg_fr, base: *const pg_g1_affine, n: u64, out: *mut pg_g1_affine, out_on_device: c_int) -> c_int;
     pub fn pg_g1_fixed_base_mul(ctx: *mut pg_ctx, n: u64, base: *const pg_g1_affine, scalars: *const pg_fr, out: *mut pg_g1_affine,

@@ -210,6 +210,32 @@ impl BatchComposer {
         })?;
         Ok((z, closing))
     }
+    /// Preprocessing's selector polynomials q_m q_l q_r q_o q_4 q_c q_arith q_range (padding rows zero) over the domain 2^log_n,
+    /// evaluations or (`coefficients`) their ifft: eight vectors of 2^log_n scalars.
+    pub fn selector_polynomials(&mut self, log_n: u32, coefficients: bool) -> Result<Vec<Vec<BlsScalar>>, EngineError> {
+        let n = 1usize << log_n;
+        let form = if coefficients { sys::PG_FORM_COEFFICIENTS } else { sys::PG_FORM_EVALUATIONS };
+        let mut flat = vec![BlsScalar::zero(); 8 * n];
+        self.ok(unsafe { sys::pg_selector_polynomials(self.ctx, log_n, form, flat.as_mut_ptr() as *mut sys::pg_fr, 0) })?;
+        Ok(flat.chunks(n).map(|c| c.to_vec()).collect())
+    }
+    /// `construct_dense_pi_vec` padded to 2^log_n, or (`coefficients`) PI(X).
+    pub fn public_input_polynomial(&mut self, log_n: u32, coefficients: bool) -> Result<Vec<BlsScalar>, EngineError> {
+        let form = if coefficients { sys::PG_FORM_COEFFICIENTS } else { sys::PG_FORM_EVALUATIONS };
+        let mut pi = vec![BlsScalar::zero(); 1usize << log_n];
+        self.ok(unsafe { sys::pg_public_input_polynomial(self.ctx, log_n, form, pi.as_mut_ptr() as *mut sys::pg_fr, 0) })?;
+        Ok(pi)
+    }
+    /// Prover round 3: t_1 .. t_4 (`split_tx_poly`), four vectors of 2^log_n coefficients, for the transcript's alpha, beta, gamma
+    /// and range separation challenge; log_n <= 30.
+    pub fn quotient(&mut self, log_n: u32, alpha: &BlsScalar, beta: &BlsScalar, gamma: &BlsScalar, range_challenge: &BlsScalar)
+                    -> Result<Vec<Vec<BlsScalar>>, EngineError> {
+        let n = 1usize << log_n;
+        let mut flat = vec![BlsScalar::zero(); 4 * n];
+        let p = |x: &BlsScalar| x as *const BlsScalar as *const sys::pg_fr;
+        self.ok(unsafe { sys::pg_quotient(self.ctx, log_n, p(alpha), p(beta), p(gamma), p(range_challenge), flat.as_mut_ptr() as *mut sys::pg_fr, 0) })?;
+        Ok(flat.chunks(n).map(|c| c.to_vec()).collect())
+    }
     /// Prover round 1, second half: `commit_key.commit(&w_l_poly)` .. `w_4`.  `powers_of_g` are the CommitKey's G1Affine
     /// powers in the layout of `sys::pg_g1_affine` (x, y Montgomery limbs; all-zero = infinity).
     pub fn commit_wire_polynomials(&mut self, log_n: u32, powers_of_g: &[sys::pg_g1_affine]) -> Result<[sys::pg_g1_affine; 4], EngineError> {

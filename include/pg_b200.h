@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define PG_B200_ABI_VERSION 4
+#define PG_B200_ABI_VERSION 5
 
 /* BlsScalar: ref:src/allocated_scalar.rs:9-12 (dusk_plonk::bls12_381::BlsScalar) */
 typedef struct pg_fr { uint64_t l[4]; } pg_fr;
@@ -335,6 +335,34 @@ int pg_permutation_z(pg_ctx *ctx, uint32_t log_n, const pg_fr *beta, const pg_fr
                      pg_fr *closing);
 int pg_permutation_z_rows(pg_ctx *ctx, uint32_t log_n, uint64_t n, const pg_fr *w_val, const uint64_t *sigma, int on_device,
                           const pg_fr *beta, const pg_fr *gamma, int form, pg_fr *dst, int dst_on_device, pg_fr *closing);
+
+/* ---- quotient polynomial (SURVEY.md section 8f item 2, continued) ------------------------------------------------------------
+ * Preprocessing's selector and public-input polynomials and round 3 of Prover::prove [DEP dusk-plonk 0.8 src/proof_system/
+ * quotient_poly.rs (compute, compute_circuit_satisfiability_equation, compute_permutation_checks, split_tx_poly), recalled like
+ * the rest of [DEP]: parity unpinned].  H = <w> of size N = 2^log_n as above; rows n_rows .. N are padding with zero wires,
+ * zero selectors (q_arith included) and zero PI (pad(), recalled).
+ * pg_selector_polynomials: q_m q_l q_r q_o q_4 q_c q_arith q_range of rows 0 .. N, 8 x N column-major, PG_FORM_EVALUATIONS or the
+ *   domain.ifft of each (PG_FORM_COEFFICIENTS).  q_logic, q_fixed_group_add and q_variable_group_add are 0 on every row (see
+ *   pg_materialize_rows): their polynomials and widget terms vanish.
+ * pg_public_input_polynomial: the dense public inputs (construct_dense_pi_vec) padded to N, or their ifft PI(X): N scalars.
+ * pg_quotient: with the caller's challenges alpha, beta, gamma and the range separation challenge rho (host pointers to one scalar
+ *   each; the transcript is not built), kappa = rho^2, Delta(f) = f(f-1)(f-2)(f-3), k = (1, 7, 13, 17), L_1(X) = (X^N - 1)/(N(X - 1)),
+ *   z(X) = pg_permutation_z's polynomial for the same beta, gamma, and at every point x of the coset g*<zeta> (zeta^4 = w, g = 7 =
+ *   dusk-bls12_381 GENERATOR; EvaluationDomain::coset_fft of the 4N domain):
+ *     arith = q_arith (q_m a b + q_l a + q_r b + q_o c + q_4 d + q_c) + PI                 (PI outside the q_arith factor)
+ *     range = rho q_range (Delta(c - 4d) + kappa Delta(b - 4c) + kappa^2 Delta(a - 4b) + kappa^3 Delta(d(xw) - 4a))
+ *     perm  = alpha z(x) prod_w (v_w + beta k_w x + gamma) - alpha z(xw) prod_w (v_w + beta sigma_w(x) + gamma) + alpha^2 L_1(x) (z(x) - 1)
+ *     t(x)  = (arith + range + perm) / (x^N - 1)
+ *   With no blinding deg t <= 4N - 5 on an honest composer.  dst: t_1 = t[0 .. N), t_2 = t[N .. 2N), t_3, t_4 (split_tx_poly), 4 x N
+ *   coefficients column-major.  The call does not judge the witness: on a composer that violates a gate or a copy constraint it
+ *   returns PG_OK and a t whose top coefficients are not zero (a verifier rejects it), like the reference's prover.
+ * All three: PG_ERR_ARG when 2^log_n < the circuit size or a null buffer; PG_ERR_STATE on a ctx whose communicator has more than one
+ *   rank.  pg_quotient also: PG_ERR_ARG when log_n > 30 (the 4N coset needs 2-adicity log_n + 2 <= 32), an unreduced challenge, or a
+ *   zero z denominator (from the z computation it makes; pg_last_error names the row).  They synchronise the ctx stream. */
+int pg_selector_polynomials(pg_ctx *ctx, uint32_t log_n, int form, pg_fr *dst, int dst_on_device);
+int pg_public_input_polynomial(pg_ctx *ctx, uint32_t log_n, int form, pg_fr *dst, int dst_on_device);
+int pg_quotient(pg_ctx *ctx, uint32_t log_n, const pg_fr *alpha, const pg_fr *beta, const pg_fr *gamma, const pg_fr *range_challenge,
+                pg_fr *dst, int dst_on_device);
 
 /* ---- commitments (SURVEY.md section 8f item 2, second half) -----------------------------------------------------------------
  * KZG commitments of coefficient vectors in the BLS12-381 group G1 [DEP dusk-plonk 0.8 CommitKey::commit =

@@ -448,6 +448,41 @@ class StandardComposer:
             head = (n, w.ctypes.data_as(C.c_void_p), s.ctypes.data_as(C.c_void_p), 0)
         return self._z_call(self._L.pg_permutation_z_rows, "pg_permutation_z_rows", log_n, head, beta, gamma, form, out)
 
+    # -- quotient polynomial: preprocessing's selector / public-input polynomials and prover round 3's t(X) ([DEP] quotient_poly.rs)
+    def _columns(self, fn, what, cols, log_n, form, out):
+        log_n = self._domain(log_n)
+        if out is not None:
+            self._ok(fn(self._ctx, log_n, form, C.c_void_p(out.data_ptr()), 1), what)
+            return out
+        dst = np.empty((cols, 1 << log_n, 4), dtype=np.uint64)
+        self._ok(fn(self._ctx, log_n, form, dst.ctypes.data_as(C.c_void_p), 0), what)
+        return dst
+
+    def selector_polynomials(self, log_n: int | None = None, form: int = FORM_EVALUATIONS, out=None):
+        """q_m q_l q_r q_o q_4 q_c q_arith q_range over the domain 2^log_n (padding rows zero): (8, 2^log_n, 4) uint64 evaluations
+        or coefficients (host array, or written to the device tensor `out`)."""
+        return self._columns(self._L.pg_selector_polynomials, "pg_selector_polynomials", 8, log_n, form, out)
+
+    def public_input_polynomial(self, log_n: int | None = None, form: int = FORM_EVALUATIONS, out=None):
+        """The dense public-input vector padded to 2^log_n, or PI(X)'s coefficients: (2^log_n, 4) uint64 (or the device tensor `out`)."""
+        r = self._columns(self._L.pg_public_input_polynomial, "pg_public_input_polynomial", 1, log_n, form, out)
+        return r if out is not None else r[0]
+
+    def quotient(self, alpha, beta, gamma, range_challenge, log_n: int | None = None, out=None):
+        """Prover round 3: t_1 .. t_4, (4, 2^log_n, 4) uint64 coefficients (or written to the device tensor `out`); the challenges
+        are one Montgomery scalar each.  log_n <= 30."""
+        log_n = self._domain(log_n)
+        if log_n > 30:
+            raise EngineError(-2, "pg_quotient", f"log_n = {log_n}: the 4N coset needs 2-adicity log_n + 2 <= 32")
+        ch = [np.ascontiguousarray(x, dtype=np.uint64).reshape(4) for x in (alpha, beta, gamma, range_challenge)]
+        vp = lambda x: x.ctypes.data_as(C.c_void_p)
+        if out is not None:
+            self._ok(self._L.pg_quotient(self._ctx, log_n, *map(vp, ch), C.c_void_p(out.data_ptr()), 1), "pg_quotient")
+            return out
+        dst = np.empty((4, 1 << log_n, 4), dtype=np.uint64)
+        self._ok(self._L.pg_quotient(self._ctx, log_n, *map(vp, ch), vp(dst), 0), "pg_quotient")
+        return dst
+
     # -- commitments: G1 multi-scalar multiplication, SRS powers, wire-polynomial commitments ([DEP] dusk-plonk 0.8 / dusk-bls12_381)
     @staticmethod
     def _points(x):

@@ -1027,6 +1027,84 @@ struct PermRatioHook {
     PG_HD static void post(const Args& a, uint64_t i, const Fr&, const Fr& den_inv) { aos_store(a.ratio, i, fr_mul(aos_load(a.ratio, i), den_inv)); }
 };
 
+// ---------------------------------------------------------------------------------------------------- quotient polynomial
+// [DEP] dusk-plonk 0.8 quotient_poly.rs (compute_circuit_satisfiability_equation + compute_permutation_checks), recalled.  The 4N
+// coset g*<zeta> is taken as four size-N sub-cosets h_j*H, h_j = g*zeta^j: point k of sub-coset j is x = h_j * w^k, and x*w is point
+// k+1 (mod N) of the same sub-coset.  Evaluation vectors, N scalars each, in this order (QV_*); the first QV_COEF are coefficient
+// vectors too (Engine::quotient), the last one is alpha^2 * L_1 (coset FFT of the constant coefficient vector alpha^2 / N).
+enum : uint32_t { QV_W = 0, QV_Z = 4, QV_S = 5, QV_QM = 9, QV_QL, QV_QR, QV_QO, QV_Q4, QV_QC, QV_QARITH, QV_QRANGE, QV_PI, QV_COEF, QV_L1 = QV_COEF, QV_EV };
+PG_HD Fr quot_delta(const Fr& f, const Fr& two, const Fr& three) {       // f(f-1)(f-2)(f-3) = u(u+2), u = f(f-3)
+    const Fr u = fr_mul(f, fr_sub(f, three));
+    return fr_mul(u, fr_add(u, two));
+}
+PG_HD Fr quot_times4(const Fr& x) { const Fr y = fr_add(x, x); return fr_add(y, y); }
+// t(x) on sub-coset j: (arith + range + perm) / (x^N - 1), 39 Montgomery multiplications per point with the range widget, 26
+// without.  has_pi / has_range are decided on the composer's row templates (no PI parameter / no range-widget row: the polynomial
+// is zero), never on witness values.
+struct QuotientBody {
+    struct Args { const uint4* ev; uint64_t n; const uint4* tw; uint32_t log_n; int has_pi, has_range;
+                  Fr bkh[4];      /* beta * k_w * h_j */
+                  Fr beta, gamma, alpha, rho, kappa, zh_inv, two, three; uint4* out; };
+    PG_HD static Fr ld(const Args& a, uint32_t v, uint64_t k) { return aos_load(a.ev, (uint64_t)v * a.n + k); }
+    PG_HD static void run(const Args& a, uint64_t k) {
+        const uint64_t kn = (k + 1) & (a.n - 1);
+        const Fr w_a = ld(a, QV_W, k), w_b = ld(a, QV_W + 1, k), w_c = ld(a, QV_W + 2, k), w_d = ld(a, QV_W + 3, k);
+        // arithmetic widget: q_arith * (q_m a b + q_l a + q_r b + q_o c + q_4 d + q_c) + PI
+        Fr g = fr_mul(fr_mul(ld(a, QV_QM, k), w_a), w_b);
+        g = fr_add(g, fr_mul(ld(a, QV_QL, k), w_a));
+        g = fr_add(g, fr_mul(ld(a, QV_QR, k), w_b));
+        g = fr_add(g, fr_mul(ld(a, QV_QO, k), w_c));
+        g = fr_add(g, fr_mul(ld(a, QV_Q4, k), w_d));
+        g = fr_add(g, ld(a, QV_QC, k));
+        Fr t = fr_mul(ld(a, QV_QARITH, k), g);
+        if (a.has_pi) t = fr_add(t, ld(a, QV_PI, k));
+        // range widget: rho * q_range * (D(c-4d) + kappa D(b-4c) + kappa^2 D(a-4b) + kappa^3 D(d(xw)-4a)), Horner in kappa
+        if (a.has_range) {
+            Fr s = quot_delta(fr_sub(ld(a, QV_W + 3, kn), quot_times4(w_a)), a.two, a.three);
+            s = fr_add(fr_mul(s, a.kappa), quot_delta(fr_sub(w_a, quot_times4(w_b)), a.two, a.three));
+            s = fr_add(fr_mul(s, a.kappa), quot_delta(fr_sub(w_b, quot_times4(w_c)), a.two, a.three));
+            s = fr_add(fr_mul(s, a.kappa), quot_delta(fr_sub(w_c, quot_times4(w_d)), a.two, a.three));
+            t = fr_add(t, fr_mul(fr_mul(a.rho, ld(a, QV_QRANGE, k)), s));
+        }
+        // permutation: alpha (z(x) prod_w (v_w + beta k_w x + gamma) - z(xw) prod_w (v_w + beta sigma_w(x) + gamma)) + alpha^2 L_1(x) (z(x) - 1)
+        const Fr wk = domain_pow(a.tw, a.log_n, k);
+        const Fr v[4] = {w_a, w_b, w_c, w_d};
+        Fr num = fr_add(fr_add(v[0], fr_mul(a.bkh[0], wk)), a.gamma);
+        Fr den = fr_add(fr_add(v[0], fr_mul(a.beta, ld(a, QV_S, k))), a.gamma);
+#pragma unroll
+        for (uint32_t w = 1; w < 4; w++) {
+            num = fr_mul(num, fr_add(fr_add(v[w], fr_mul(a.bkh[w], wk)), a.gamma));
+            den = fr_mul(den, fr_add(fr_add(v[w], fr_mul(a.beta, ld(a, QV_S + w, k))), a.gamma));
+        }
+        const Fr z = ld(a, QV_Z, k);
+        const Fr p = fr_mul(a.alpha, fr_sub(fr_mul(z, num), fr_mul(ld(a, QV_Z, kn), den)));
+        t = fr_add(t, fr_add(p, fr_mul(ld(a, QV_L1, k), fr_sub(z, fr_one()))));
+        aos_store(a.out, k, fr_mul(t, a.zh_inv));                                 // / Z_H(x) = x^N - 1, one constant per sub-coset
+    }
+};
+// t's coefficients from the inverse size-N transforms c_j of the four sub-cosets' values (in place, t[j*n + m] = c_j[m]):
+//   c_j[m] = zeta^(jm) * sum_r iota^(jr) * t_(m+rN) g^(m+rN),  iota = zeta^N,
+// so with e_j = c_j[m] * h_j^-m (h_j^-m = g^-m zeta^-jm, from two-level tables) a 4-point inverse DFT over j gives
+// t_(m+rN) = (1/4) g^-rN * sum_j iota^-jr e_j, written to t[r*n + m]: split_tx_poly's t_1 .. t_4 directly.
+struct QuotientSplitBody {
+    struct Args { uint4* t; uint64_t n; const uint4* inv_tab[4]; uint32_t log_lo; Fr iota_inv; Fr scale[4]; };
+    PG_HD static void run(const Args& a, uint64_t m) {
+        Fr e[4];
+#pragma unroll
+        for (uint32_t j = 0; j < 4; j++) e[j] = fr_mul(aos_load(a.t, (uint64_t)j * a.n + m), pow_table_at(a.inv_tab[j], a.log_lo, m));
+        const Fr s02 = fr_add(e[0], e[2]), d02 = fr_sub(e[0], e[2]);
+        const Fr s13 = fr_add(e[1], e[3]), d13 = fr_mul(a.iota_inv, fr_sub(e[1], e[3]));
+        const Fr y[4] = {fr_add(s02, s13), fr_add(d02, d13), fr_sub(s02, s13), fr_sub(d02, d13)};
+#pragma unroll
+        for (uint32_t r = 0; r < 4; r++) aos_store(a.t, (uint64_t)r * a.n + m, fr_mul(y[r], a.scale[r]));
+    }
+};
+// data[i] = v
+struct FillBody {
+    struct Args { uint4* data; Fr v; uint64_t n; };
+    PG_HD static void run(const Args& a, uint64_t i) { aos_store(a.data, i, a.v); }
+};
+
 // ---------------------------------------------------------------------------------------------------- synthetic inputs
 PG_HD uint64_t splitmix64_at(uint64_t seed, uint64_t index1) {   // output number index1 (1-based) of SplitMix64(seed)
     uint64_t z = seed + index1 * 0x9E3779B97F4A7C15ull;

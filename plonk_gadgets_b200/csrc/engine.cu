@@ -67,6 +67,7 @@ public:
         check_shape = cfg.check_shape < (uint32_t)CHECK_SHAPES ? (int)cfg.check_shape : 0;
         PG_CUDA(cudaFuncSetAttribute(k_ntt_pass<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 << NTT_MAX_LOG_TILE));
         PG_CUDA(cudaFuncSetAttribute(k_ntt_pass<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 << NTT_MAX_LOG_TILE));
+        PG_CUDA(cudaFuncSetAttribute(k_ntt_coset_pass, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 << NTT_MAX_LOG_TILE));
         PG_CUDA(cudaFuncSetAttribute(k_check_rowpar<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         PG_CUDA(cudaFuncSetAttribute(k_check_rowpar<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         if (!set_check_attrs<0>() || !set_check_attrs<1>() || !set_check_attrs<2>() || !set_check_attrs<3>() || !set_check_attrs<4>()) return false;
@@ -420,10 +421,11 @@ public:
     bool run_ntt_pass(const NttPassArgs& a, uint64_t n_blocks) {
         const size_t smem = (size_t)32 << (a.s + a.log_c);
         tic(CLS_OTHER, 0);
-        if (a.inverse) k_ntt_pass<true><<<(unsigned)n_blocks, NTT_THREADS, smem, stream>>>(a);
+        if (a.shift) k_ntt_coset_pass<<<(unsigned)n_blocks, NTT_THREADS, smem, stream>>>(a);
+        else if (a.inverse) k_ntt_pass<true><<<(unsigned)n_blocks, NTT_THREADS, smem, stream>>>(a);
         else k_ntt_pass<false><<<(unsigned)n_blocks, NTT_THREADS, smem, stream>>>(a);
         toc();
-        return launched("k_ntt_pass");
+        return launched(a.shift ? "k_ntt_coset_pass" : "k_ntt_pass");
     }
     // exclusive prefix product (scan.cuh) of n scalars; *total = product of all; scratch: fr_scan_scratch(n) scalars
     bool run_fr_scan(const uint4* in, uint4* out, uint64_t n, uint4* total, uint4* scratch) {

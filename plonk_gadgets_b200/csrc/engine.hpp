@@ -1122,8 +1122,13 @@ public:
     // Transform of `data` in place.  Transforms of more than 2^11 points go through a scratch vector of the same size (first
     // pass data -> scratch with the bit reversal folded into its loads, last pass scratch -> data); it is only touched by
     // kernels on the engine's stream, so it goes back to the pool as soon as they are enqueued.
-    int ntt_inplace(uint4* data, uint32_t log_n, bool inverse) {
-        if (log_n == 0) return PG_OK;                                    // one element: the transform is the identity
+    int ntt_inplace(uint4* data, uint32_t log_n, bool inverse) { return ntt_transform(data, data, log_n, inverse, nullptr); }
+    // The same from src to dst (the same buffer, or two that do not overlap).  shift_tab != nullptr (forward only): the coset
+    // transform of EvaluationDomain::coset_fft, source element m multiplied by h^m from pow_table_host's two-level table of h.
+    int ntt_transform(const uint4* src, uint4* data, uint32_t log_n, bool inverse, const uint4* shift_tab) {
+        if (shift_tab && inverse) return fail(PG_ERR_ARG, "ntt: a coset shift applies to the forward transform only");
+        if (log_n == 0)                                                  // one element: the transform is the identity (h^0 = 1)
+            return src == data || be.d2d(data, src, sizeof(pg_fr)) ? PG_OK : fail(PG_ERR_CUDA, "device copy");
         int rc = ntt_twiddles(log_n);
         if (rc) return rc;
         const uint64_t n = 1ull << log_n;
@@ -1135,10 +1140,11 @@ public:
         for (uint32_t p = 0; p < plan.n_pass; p++) {
             NttPassArgs a; memset(&a, 0, sizeof(a));
             const bool first = p == 0, last = p + 1 == plan.n_pass;
-            a.src = first ? data : work;                                 // first pass: gather through the bit reversal, scale
+            a.src = first ? src : work;                                  // first pass: gather through the bit reversal, scale / shift
             a.dst = last ? data : work;                                  // last pass: back to the caller's buffer
             a.tw = ntt_tw; a.log_n = log_n; a.t0 = plan.t0[p]; a.s = plan.s[p]; a.log_c = plan.log_c[p];
             a.inverse = inverse ? 1 : 0; a.bitrev = first ? 1 : 0; a.scale = first && inverse ? 1 : 0; a.factor = factor;
+            if (first && shift_tab) { a.shift = 1; a.shift_tab = shift_tab; a.shift_log_lo = pow_table_log_lo(log_n); }
             if (!be.run_ntt_pass(a, n >> (plan.s[p] + plan.log_c[p]))) { dfree(work); return fail(PG_ERR_CUDA, "NTT pass kernel"); }
         }
         dfree(work);
@@ -1411,6 +1417,134 @@ public:
         }
         if (closing && (rc = deliver(closing, tot, sizeof(pg_fr), 0))) return rc;
         if (!dst_on_device && (rc = deliver(dst, z, n * sizeof(pg_fr), 0))) return rc;
+        release_scratch_from(mark);
+        return PG_OK;
+    }
+
+    // ------------------------------------------------------------------------------------------------ quotient polynomial
+    // Preprocessing's selector and public-input polynomials and prover round 3's t(X) [DEP dusk-plonk 0.8 quotient_poly.rs, recalled];
+    // bodies.cuh QuotientBody / QuotientSplitBody, ntt.cuh k_ntt_coset_pass.
+    // the eight selector columns q_m q_l q_r q_o q_4 q_c q_arith q_range (padding rows 0) in 8 columns of 2^log_n, optionally ifft'd
+    int selector_polynomials(uint32_t log_n, int form, pg_fr* dst, int dst_on_device) {
+        int rc;
+        if ((rc = perm_unsharded("selector_polynomials")) || (rc = perm_domain("selector_polynomials", log_n, n_rows, form))) return rc;
+        if (!dst) return fail(PG_ERR_ARG, "selector_polynomials: null buffer");
+        const uint64_t n = 1ull << log_n; const size_t bytes = 8 * n * sizeof(pg_fr);
+        const size_t mark = scratch.size();
+        uint4* buf = reinterpret_cast<uint4*>(dst);
+        if (!dst_on_device) { buf = (uint4*)dalloc(bytes); if (!buf) return fail(PG_ERR_OOM, "selector buffer"); scratch.push_back(buf); }
+        if ((rc = materialize_dev(0, n_rows, n, nullptr, nullptr, buf, nullptr))) return rc;          // q_m .. q_c
+        GateSelBody::Args g{d_segs, (uint32_t)dsegs.size(), 0, n_rows, buf + 2 * 6 * n, buf + 2 * 7 * n};  // q_arith, q_range
+        if (!be.template run_simple<GateSelBody>(g, n_rows, CLS_OTHER)) return fail(PG_ERR_CUDA, "gate selector kernel");
+        for (uint64_t c = 0; c < 8; c++) {
+            uint4* col = buf + 2 * c * n;
+            NttZeroBody::Args z{col, n_rows, n - n_rows};
+            if (n > n_rows && !be.template run_simple<NttZeroBody>(z, z.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "padding kernel");
+            if (form == PG_FORM_COEFFICIENTS && (rc = ntt_inplace(col, log_n, true))) return rc;
+        }
+        if (dst_on_device) return PG_OK;
+        rc = deliver(dst, buf, bytes, 0);
+        release_scratch_from(mark);
+        return rc;
+    }
+    // construct_dense_pi_vec padded with zeros to 2^log_n, optionally ifft'd
+    int public_input_polynomial(uint32_t log_n, int form, pg_fr* dst, int dst_on_device) {
+        int rc;
+        if ((rc = perm_unsharded("public_input_polynomial")) || (rc = perm_domain("public_input_polynomial", log_n, n_rows, form))) return rc;
+        if (!dst) return fail(PG_ERR_ARG, "public_input_polynomial: null buffer");
+        const uint64_t n = 1ull << log_n; const size_t bytes = n * sizeof(pg_fr);
+        const size_t mark = scratch.size();
+        uint4* buf = reinterpret_cast<uint4*>(dst);
+        if (!dst_on_device) { buf = (uint4*)dalloc(bytes); if (!buf) return fail(PG_ERR_OOM, "public input buffer"); scratch.push_back(buf); }
+        if ((rc = materialize_dev(0, n_rows, n, nullptr, nullptr, nullptr, buf))) return rc;
+        NttZeroBody::Args z{buf, n_rows, n - n_rows};
+        if (n > n_rows && !be.template run_simple<NttZeroBody>(z, z.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "padding kernel");
+        if (form == PG_FORM_COEFFICIENTS && (rc = ntt_inplace(buf, log_n, true))) return rc;
+        if (dst_on_device) return PG_OK;
+        rc = deliver(dst, buf, bytes, 0);
+        release_scratch_from(mark);
+        return rc;
+    }
+    static Fr fr_small(uint64_t v) { Fr raw = fr_zero(); raw.v[0] = (uint32_t)v; raw.v[1] = (uint32_t)(v >> 32); return fr_to_mont(raw); }
+    static Fr fr_pow2k(Fr x, uint32_t k) { for (uint32_t i = 0; i < k; i++) x = fr_sqr(x); return x; }     // x^(2^k)
+    // Round 3: t_1 .. t_4 (4 columns of N = 2^log_n coefficients).  Coefficient vectors of the wires, z, sigma, the selectors and PI
+    // (QV_* order), then per sub-coset j: coset FFTs of each (shift h_j = g zeta^j) and of alpha^2 / N (= alpha^2 L_1), the
+    // numerator / Z_H pointwise; then an inverse size-N transform per sub-coset and the split.
+    int quotient(uint32_t log_n, const pg_fr* alpha, const pg_fr* beta, const pg_fr* gamma, const pg_fr* rho, pg_fr* dst, int dst_on_device) {
+        int rc;
+        if ((rc = perm_unsharded("quotient"))) return rc;
+        if (log_n > NTT_TWO_ADICITY - 2 || (1ull << log_n) < n_rows)
+            return fail(PG_ERR_ARG, "quotient: domain smaller than the circuit, or larger than 2^30 (the 4N coset needs 2-adicity log_n + 2 <= 32)");
+        if (!alpha || !beta || !gamma || !rho || !dst) return fail(PG_ERR_ARG, "quotient: null argument");
+        if (!host_reduced(*alpha) || !host_reduced(*beta) || !host_reduced(*gamma) || !host_reduced(*rho))
+            return fail(PG_ERR_ARG, "quotient: alpha / beta / gamma / range_challenge not fully reduced (>= q)");
+        // polynomials that are zero by the composer's structure: no row template has a public input / a range-widget row
+        bool has_pi = false, has_range = false;
+        for (const Segment& s : segs) {
+            if (!s.n_inst) continue;
+            for (const RowT& r : s.t.rows) { has_range = has_range || r.gate == GATE_RANGE; has_pi = has_pi || r.pi_param >= 0 || r.pi_sel != POOL_ZERO; }
+        }
+        const uint64_t n = 1ull << log_n;
+        const size_t mark = scratch.size();
+        auto col = [n](uint4* base, uint32_t v) { return base + 2 * (uint64_t)v * n; };
+        uint4* coef = (uint4*)dalloc(QV_COEF * n * sizeof(pg_fr)); if (!coef) return fail(PG_ERR_OOM, "quotient coefficient vectors");
+        scratch.push_back(coef);
+        if ((rc = wire_polynomials(log_n, (pg_fr*)col(coef, QV_W), 1))) return rc;
+        if ((rc = permutation_z(log_n, beta, gamma, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_Z), 1, nullptr))) return rc;
+        if ((rc = sigma_polynomials(log_n, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_S), 1))) return rc;
+        if ((rc = selector_polynomials(log_n, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_QM), 1))) return rc;
+        if (has_pi && (rc = public_input_polynomial(log_n, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_PI), 1))) return rc;
+        uint4* ev = (uint4*)dalloc(QV_EV * n * sizeof(pg_fr)); if (!ev) return fail(PG_ERR_OOM, "quotient evaluation vectors");
+        scratch.push_back(ev);
+        uint4* out = reinterpret_cast<uint4*>(dst);
+        if (!dst_on_device) { out = (uint4*)dalloc(4 * n * sizeof(pg_fr)); if (!out) return fail(PG_ERR_OOM, "quotient buffer"); scratch.push_back(out); }
+        // constants: zeta generates the 4N-th roots (zeta^4 = w), iota = zeta^N, g = 7 (dusk-bls12_381 GENERATOR), h_j = g zeta^j
+        const Fr zeta = fr_pow2k(fr_root_of_unity(), NTT_TWO_ADICITY - log_n - 2), iota = fr_pow2k(zeta, log_n);
+        const Fr g = fr_small(7), g_n = fr_pow2k(g, log_n), n_inv = fr_inv_fermat(fr_small(n));
+        const Fr al = fr_from_pg(*alpha), be_ = fr_from_pg(*beta), ga = fr_from_pg(*gamma), rh = fr_from_pg(*rho);
+        Fr h[4], iota_j[4];
+        h[0] = g; iota_j[0] = fr_one();
+        for (int j = 1; j < 4; j++) { h[j] = fr_mul(h[j - 1], zeta); iota_j[j] = fr_mul(iota_j[j - 1], iota); }
+        // two-level power tables of h_j (coset FFTs) and h_j^-1 (split): table j at tabs + 2 * j * entries, j = 0..7
+        const uint64_t entries = pow_table_entries(log_n);
+        std::vector<Fr> host_tabs(8 * entries);
+        for (int j = 0; j < 4; j++) {
+            pow_table_host(h[j], log_n, host_tabs.data() + j * entries);
+            pow_table_host(fr_inv_fermat(h[j]), log_n, host_tabs.data() + (4 + j) * entries);
+        }
+        uint4* tabs = (uint4*)dalloc(host_tabs.size() * sizeof(pg_fr)); if (!tabs) return fail(PG_ERR_OOM, "coset power tables");
+        scratch.push_back(tabs);
+        if (!be.h2d(tabs, host_tabs.data(), host_tabs.size() * sizeof(pg_fr))) return fail(PG_ERR_CUDA, "coset power table copy");
+        if ((rc = ntt_twiddles(log_n))) return rc;
+        QuotientBody::Args q; memset(&q, 0, sizeof(q));
+        q.ev = ev; q.n = n; q.tw = ntt_tw; q.log_n = log_n; q.has_pi = has_pi; q.has_range = has_range;
+        q.beta = be_; q.gamma = ga; q.alpha = al; q.rho = rh; q.kappa = fr_sqr(rh); q.two = fr_small(2); q.three = fr_small(3);
+        const Fr l1_coef = fr_mul(fr_sqr(al), n_inv);                         // alpha^2 L_1(X) = alpha^2 / N * sum_{i<N} X^i
+        for (uint32_t j = 0; j < 4; j++) {
+            const uint4* tab = tabs + 2 * (uint64_t)j * entries;
+            for (uint32_t v = 0; v < QV_COEF; v++) {
+                if ((v == QV_PI && !has_pi) || (v == QV_QRANGE && !has_range)) continue;
+                if ((rc = ntt_transform(col(coef, v), col(ev, v), log_n, false, tab))) return rc;
+            }
+            FillBody::Args f{col(ev, QV_L1), l1_coef, n};
+            if (!be.template run_simple<FillBody>(f, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "fill kernel");
+            if ((rc = ntt_transform(col(ev, QV_L1), col(ev, QV_L1), log_n, false, tab))) return rc;
+            for (uint32_t w = 0; w < 4; w++) q.bkh[w] = fr_mul(fr_mul(be_, perm_coset(w)), h[j]);
+            q.zh_inv = fr_inv_fermat(fr_sub(fr_mul(g_n, iota_j[j]), fr_one()));    // x^N - 1 = g^N iota^j - 1 on all of sub-coset j
+            q.out = col(out, j);
+            if (!be.template run_simple<QuotientBody>(q, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "quotient kernel");
+        }
+        for (uint32_t j = 0; j < 4; j++)
+            if ((rc = ntt_inplace(col(out, j), log_n, true))) return rc;
+        QuotientSplitBody::Args s; memset(&s, 0, sizeof(s));
+        s.t = out; s.n = n; s.log_lo = pow_table_log_lo(log_n); s.iota_inv = fr_inv_fermat(iota);
+        const Fr g_n_inv = fr_inv_fermat(g_n);
+        s.scale[0] = fr_inv_fermat(fr_small(4));                                          // (1/4) g^-rN
+        for (int r = 1; r < 4; r++) s.scale[r] = fr_mul(s.scale[r - 1], g_n_inv);
+        for (int j = 0; j < 4; j++) s.inv_tab[j] = tabs + 2 * (uint64_t)(4 + j) * entries;
+        if (!be.template run_simple<QuotientSplitBody>(s, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "quotient split kernel");
+        if (!dst_on_device) { if ((rc = deliver(dst, out, 4 * n * sizeof(pg_fr), 0))) return rc; }
+        else if (!be.sync()) return fail(PG_ERR_CUDA, "sync");                            // the coefficient and evaluation vectors go back to the pool
         release_scratch_from(mark);
         return PG_OK;
     }

@@ -76,7 +76,27 @@ struct NttZeroBody {
 // of a transform (t0 == 0) can gather its input through the bit-reversal permutation (bitrev != 0) and multiply it by
 // `factor` (scale != 0: the n^-1 of the inverse transform): no separate permutation pass.  Such a pass must not run in place
 // unless it is a single block.
-struct NttPassArgs { const uint4* src; uint4* dst; const uint4* tw; uint32_t log_n, t0, s, log_c; int inverse; int bitrev; int scale; Fr factor; };
+// shift != 0 (forward transforms only: EvaluationDomain::coset_fft): the first pass also multiplies source element m by h^m, read
+// from a two-level table, shift_tab[m & (2^shift_log_lo - 1)] * shift_tab[2^shift_log_lo + (m >> shift_log_lo)] (pow_table_host);
+// such a pass runs as k_ntt_coset_pass so that k_ntt_pass is compiled without it.
+struct NttPassArgs { const uint4* src; uint4* dst; const uint4* tw; uint32_t log_n, t0, s, log_c; int inverse; int bitrev; int scale; Fr factor;
+                     int shift; uint32_t shift_log_lo; const uint4* shift_tab; };
+
+// h^m for m < 2^log_n from a two-level table of h: [h^0 .. h^(L-1)] then [h^0, h^L, h^(2L) ..], L = 2^log_lo
+PG_HD Fr pow_table_at(const uint4* tab, uint32_t log_lo, uint64_t m) {
+    return fr_mul(aos_load(tab, m & ((1ull << log_lo) - 1ull)), aos_load(tab, (1ull << log_lo) + (m >> log_lo)));
+}
+PG_HD uint32_t pow_table_log_lo(uint32_t log_n) { return (log_n + 1) / 2; }
+PG_HD uint64_t pow_table_entries(uint32_t log_n) { const uint32_t lo = pow_table_log_lo(log_n); return (1ull << lo) + (1ull << (log_n - lo)); }
+// the table of h for exponents below 2^log_n (host code; a few thousand multiplications)
+inline void pow_table_host(Fr h, uint32_t log_n, Fr* out) {
+    const uint32_t lo = pow_table_log_lo(log_n);
+    const uint64_t L = 1ull << lo, H = 1ull << (log_n - lo);
+    Fr x = fr_one();
+    for (uint64_t i = 0; i < L; i++) { out[i] = x; x = fr_mul(x, h); }     // x = h^L afterwards
+    Fr y = fr_one();
+    for (uint64_t i = 0; i < H; i++) { out[L + i] = y; y = fr_mul(y, x); }
+}
 
 PG_HD uint64_t ntt_index(const NttPassArgs& a, uint64_t blk, uint32_t e) {
     const uint32_t c = e & ((1u << a.log_c) - 1u), v = e >> a.log_c;
@@ -169,18 +189,18 @@ __device__ __forceinline__ void ntt_stage_pair(const NttPassArgs& a, uint4* s_ti
         tile_store(s_tile, E, e0 + 2 * d, x2); tile_store(s_tile, E, e0 + 3 * d, x3);
     }
 }
-template <bool INV>
-__global__ void __launch_bounds__(NTT_THREADS, 3) k_ntt_pass(const NttPassArgs a) {
-    extern __shared__ __align__(16) uint4 s_tile[];               // [2 halves][E]
-    __shared__ uint32_t s_q[8];
+template <bool INV, bool SHIFT>
+__device__ __forceinline__ void ntt_pass_body(const NttPassArgs& a, uint4* s_tile, uint32_t* s_q) {
     const uint32_t log_e = a.s + a.log_c, E = 1u << log_e;
     const uint32_t blk = blockIdx.x;
     if (threadIdx.x < 8) s_q[threadIdx.x] = c_q[threadIdx.x];
     for (uint32_t e = threadIdx.x; e < E; e += NTT_THREADS)
     {
         const uint32_t idx = ntt_index32(a, blk, e);
-        Fr x = aos_load(a.src, a.bitrev ? (a.log_n ? __brev(idx) >> (32u - a.log_n) : 0u) : idx);
+        const uint32_t m = a.bitrev ? (a.log_n ? __brev(idx) >> (32u - a.log_n) : 0u) : idx;
+        Fr x = aos_load(a.src, m);
         if (a.scale) x = fr_mul_eo(x, a.factor);
+        if (SHIFT) x = fr_mul_eo(x, pow_table_at(a.shift_tab, a.shift_log_lo, m));
         tile_store(s_tile, E, e, x);
     }
     __syncthreads();
@@ -213,6 +233,18 @@ __global__ void __launch_bounds__(NTT_THREADS, 3) k_ntt_pass(const NttPassArgs a
     for (uint32_t e = threadIdx.x; e < E; e += NTT_THREADS)
         aos_store(a.dst, ntt_index32(a, blk, e), tile_load(s_tile, E, e));
 }
+template <bool INV>
+__global__ void __launch_bounds__(NTT_THREADS, 3) k_ntt_pass(const NttPassArgs a) {
+    extern __shared__ __align__(16) uint4 s_tile[];               // [2 halves][E]
+    __shared__ uint32_t s_q[8];
+    ntt_pass_body<INV, false>(a, s_tile, s_q);
+}
+// the first pass of a coset transform (shift != 0); the other passes of that transform are ordinary k_ntt_pass launches
+__global__ void __launch_bounds__(NTT_THREADS, 3) k_ntt_coset_pass(const NttPassArgs a) {
+    extern __shared__ __align__(16) uint4 s_tile[];
+    __shared__ uint32_t s_q[8];
+    ntt_pass_body<false, true>(a, s_tile, s_q);
+}
 #endif
 
 // the same tile schedule on the host (tests/emu backend and documentation of the kernel's data flow)
@@ -222,8 +254,10 @@ inline void ntt_pass_host(const NttPassArgs& a, uint64_t n_blocks) {
     for (uint64_t blk = 0; blk < n_blocks; blk++) {
         for (uint32_t e = 0; e < E; e++) {
             const uint64_t idx = ntt_index(a, blk, e);
-            tile[e] = aos_load(a.src, a.bitrev ? bitrev64(idx, a.log_n) : idx);
+            const uint64_t m = a.bitrev ? bitrev64(idx, a.log_n) : idx;
+            tile[e] = aos_load(a.src, m);
             if (a.scale) tile[e] = fr_mul(tile[e], a.factor);
+            if (a.shift) tile[e] = fr_mul(tile[e], pow_table_at(a.shift_tab, a.shift_log_lo, m));
         }
         for (uint32_t u = 0; u < a.s; u++)
             for (uint32_t b = 0; b < E / 2; b++) {

@@ -170,6 +170,27 @@ public:
                             reinterpret_cast<pg_fr*>(closing)), "pg_permutation_z");
         return out;
     }
+    /// preprocessing's q_m q_l q_r q_o q_4 q_c q_arith q_range over the domain 2^log_n (evaluations, or coefficients): 8 x 2^log_n scalars
+    std::vector<BlsScalar> selector_polynomials(uint32_t log_n, bool coefficients = false) {
+        std::vector<BlsScalar> out((size_t)8 << log_n);
+        ok(pg_selector_polynomials(ctx_, log_n, coefficients ? PG_FORM_COEFFICIENTS : PG_FORM_EVALUATIONS, reinterpret_cast<pg_fr*>(out.data()), 0),
+           "pg_selector_polynomials");
+        return out;
+    }
+    /// the dense public inputs padded to 2^log_n (evaluations), or PI(X) (coefficients)
+    std::vector<BlsScalar> public_input_polynomial(uint32_t log_n, bool coefficients = false) {
+        std::vector<BlsScalar> out((size_t)1 << log_n);
+        ok(pg_public_input_polynomial(ctx_, log_n, coefficients ? PG_FORM_COEFFICIENTS : PG_FORM_EVALUATIONS, reinterpret_cast<pg_fr*>(out.data()), 0),
+           "pg_public_input_polynomial");
+        return out;
+    }
+    /// prover round 3: t_1 .. t_4, 4 x 2^log_n coefficients, for the caller's alpha, beta, gamma and range separation challenge
+    std::vector<BlsScalar> quotient(uint32_t log_n, const BlsScalar& alpha, const BlsScalar& beta, const BlsScalar& gamma, const BlsScalar& range_challenge) {
+        std::vector<BlsScalar> out((size_t)4 << log_n);
+        auto p = [](const BlsScalar& x) { return reinterpret_cast<const pg_fr*>(&x); };
+        ok(pg_quotient(ctx_, log_n, p(alpha), p(beta), p(gamma), p(range_challenge), reinterpret_cast<pg_fr*>(out.data()), 0), "pg_quotient");
+        return out;
+    }
     /// EvaluationDomain::fft / ifft of 2^k scalars
     std::vector<BlsScalar> fft(const std::vector<BlsScalar>& v, bool inverse) {
         uint32_t log_n = 0; while ((1ull << log_n) < v.size()) log_n++;
