@@ -10,6 +10,17 @@ pub struct pg_fr {
     pub l: [u64; 4],
 }
 /// G1Affine { x, y } of dusk-bls12_381 without the infinity flag (all-zero = point at infinity).
+/// The evaluations of prover round 4 (include/pg_b200.h): dusk-plonk 0.8 ProofEvaluations' fields in order, then quot_eval.
+#[repr(C)]
+#[derive(Copy, Clone, Debug, Default, PartialEq, Eq)]
+pub struct pg_proof_evaluations {
+    pub a_eval: pg_fr, pub b_eval: pg_fr, pub c_eval: pg_fr, pub d_eval: pg_fr,
+    pub a_next_eval: pg_fr, pub b_next_eval: pg_fr, pub d_next_eval: pg_fr,
+    pub q_arith_eval: pg_fr, pub q_c_eval: pg_fr, pub q_l_eval: pg_fr, pub q_r_eval: pg_fr,
+    pub left_sigma_eval: pg_fr, pub right_sigma_eval: pg_fr, pub out_sigma_eval: pg_fr,
+    pub lin_poly_eval: pg_fr, pub perm_eval: pg_fr, pub quot_eval: pg_fr,
+}
+
 #[repr(C)]
 #[derive(Copy, Clone, Debug, Default, PartialEq, Eq)]
 pub struct pg_g1_affine {
@@ -161,6 +172,8 @@ extern "C" {
     pub fn pg_public_input_polynomial(ctx: *mut pg_ctx, log_n: u32, form: c_int, dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
     pub fn pg_quotient(ctx: *mut pg_ctx, log_n: u32, alpha: *const pg_fr, beta: *const pg_fr, gamma: *const pg_fr, range_challenge: *const pg_fr,
                        dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
+    pub fn pg_prover_openings(ctx: *mut pg_ctx, log_n: u32, challenges: *const pg_fr, t: *const pg_fr, t_on_device: c_int,
+                              evals: *mut pg_proof_evaluations, dst: *mut pg_fr, dst_on_device: c_int) -> c_int;
     pub fn pg_msm(ctx: *mut pg_ctx, n: u64, points: *const pg_g1_affine, scalars: *const pg_fr, out: *mut pg_g1_affine, on_device: c_int) -> c_int;
     pub fn pg_srs_powers(ctx: *mut pg_ctx, beta: *const pg_fr, base: *const pg_g1_affine, n: u64, out: *mut pg_g1_affine, out_on_device: c_int) -> c_int;
     pub fn pg_g1_fixed_base_mul(ctx: *mut pg_ctx, n: u64, base: *const pg_g1_affine, scalars: *const pg_fr, out: *mut pg_g1_affine,

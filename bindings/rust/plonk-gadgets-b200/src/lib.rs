@@ -236,6 +236,22 @@ impl BatchComposer {
         self.ok(unsafe { sys::pg_quotient(self.ctx, log_n, p(alpha), p(beta), p(gamma), p(range_challenge), flat.as_mut_ptr() as *mut sys::pg_fr, 0) })?;
         Ok(flat.chunks(n).map(|c| c.to_vec()).collect())
     }
+    /// Prover rounds 4 and 5 for round 3's t_1 .. t_4 and the transcript's alpha, beta, gamma, range separation challenge, z_challenge
+    /// and the two aggregation challenges v (opening at z) and v' (opening at z*w): the evaluations, and W_z, W_zw and r as
+    /// vectors of 2^log_n coefficients; log_n <= 30.
+    pub fn prover_openings(&mut self, log_n: u32, t: &[Vec<BlsScalar>], challenges: &[BlsScalar; 7])
+                           -> Result<(sys::pg_proof_evaluations, Vec<Vec<BlsScalar>>), EngineError> {
+        let n = 1usize << log_n;
+        assert!(t.len() == 4 && t.iter().all(|c| c.len() == n), "t: four vectors of 2^log_n coefficients");
+        let flat_t: Vec<BlsScalar> = t.iter().flatten().copied().collect();
+        let mut ev = sys::pg_proof_evaluations::default();
+        let mut flat = vec![BlsScalar::zero(); 3 * n];
+        self.ok(unsafe {
+            sys::pg_prover_openings(self.ctx, log_n, challenges.as_ptr() as *const sys::pg_fr, flat_t.as_ptr() as *const sys::pg_fr, 0, &mut ev,
+                                    flat.as_mut_ptr() as *mut sys::pg_fr, 0)
+        })?;
+        Ok((ev, flat.chunks(n).map(|c| c.to_vec()).collect()))
+    }
     /// Prover round 1, second half: `commit_key.commit(&w_l_poly)` .. `w_4`.  `powers_of_g` are the CommitKey's G1Affine
     /// powers in the layout of `sys::pg_g1_affine` (x, y Montgomery limbs; all-zero = infinity).
     pub fn commit_wire_polynomials(&mut self, log_n: u32, powers_of_g: &[sys::pg_g1_affine]) -> Result<[sys::pg_g1_affine; 4], EngineError> {

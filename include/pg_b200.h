@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define PG_B200_ABI_VERSION 5
+#define PG_B200_ABI_VERSION 6
 
 /* BlsScalar: ref:src/allocated_scalar.rs:9-12 (dusk_plonk::bls12_381::BlsScalar) */
 typedef struct pg_fr { uint64_t l[4]; } pg_fr;
@@ -364,6 +364,49 @@ int pg_public_input_polynomial(pg_ctx *ctx, uint32_t log_n, int form, pg_fr *dst
 int pg_quotient(pg_ctx *ctx, uint32_t log_n, const pg_fr *alpha, const pg_fr *beta, const pg_fr *gamma, const pg_fr *range_challenge,
                 pg_fr *dst, int dst_on_device);
 
+/* ---- openings: prover rounds 4 and 5 (SURVEY.md section 8f item 2, continued) ---------------------------------------------------
+ * [DEP dusk-plonk 0.8 Prover::prove (the evaluations, compute_quotient_opening_poly / compute_aggregate_witness), linearisation_poly::
+ * compute, the widgets' compute_linearisation and Polynomial::ruffini, recalled like the rest of [DEP]: parity unpinned.]
+ * H, N, the padding, alpha, beta, gamma, rho, kappa = rho^2, Delta and k = (1, 7, 13, 17) are those of pg_quotient; w generates H.
+ * challenges: 7 host scalars alpha beta gamma rho zeta v v' (zeta: the evaluation challenge; v, v': the aggregation challenges of the
+ * openings at zeta and at zeta*w; the transcript is not built).  t: pg_quotient's 4 x N output for the same alpha, beta, gamma, rho.
+ * Z_H(zeta) = zeta^N - 1, L_1(zeta) = Z_H(zeta) / (N (zeta - 1)).
+ * Evaluations (pg_proof_evaluations, ProofEvaluations' order, then quot_eval):
+ *   a b c d = w_l w_r w_o w_4 at zeta;  a_w b_w d_w = w_l w_r w_4 at zeta*w;  q_arith q_c q_l q_r at zeta;  sigma_1..3 at zeta;
+ *   lin = r(zeta);  perm = z(zeta*w);  quot = t_1(zeta) + zeta^N t_2(zeta) + zeta^2N t_3(zeta) + zeta^3N t_4(zeta).
+ * Linearisation polynomial (PI is not in r; the verifier adds PI(zeta)):
+ *   r(X) = q_arith (a b q_m + a q_l + b q_r + c q_o + d q_4 + q_c)
+ *        + rho (Delta(c - 4d) + kappa Delta(b - 4c) + kappa^2 Delta(a - 4b) + kappa^3 Delta(d_w - 4a)) q_range
+ *        + (alpha prod_w (v_w + beta k_w zeta + gamma) + alpha^2 L_1(zeta)) z
+ *        - alpha beta perm (a + beta sigma_1 + gamma)(b + beta sigma_2 + gamma)(c + beta sigma_3 + gamma) sigma_4
+ *   with the scalars above (v_w = a b c d), the polynomials q_*, z, sigma_4 of X.
+ * Opening witnesses, ruffini(f, p) = the quotient of f by (X - p) without the remainder (q_(N-2) = f_(N-1), q_(i-1) = f_i + p q_i),
+ * N coefficients with q_(N-1) = 0:
+ *   W_zeta   = ruffini(t_1 + zeta^N t_2 + zeta^2N t_3 + zeta^3N t_4 + v r + v^2 w_l + v^3 w_r + v^4 w_o + v^5 w_4
+ *                      + v^6 sigma_1 + v^7 sigma_2 + v^8 sigma_3, zeta)
+ *   W_zeta_w = ruffini(z + v' w_l + v'^2 w_r + v'^3 w_4, zeta*w)
+ * The quotient identity.  By pg_quotient's definition, on an honest composer t(X) Z_H(X) = arith + range + perm as polynomials, so at
+ * zeta: quot * Z_H(zeta) = arith(zeta) + range(zeta) + perm(zeta).  Substituting the evaluations, arith(zeta) + range(zeta) is r's first
+ * two lines plus PI(zeta); perm(zeta) = alpha z(zeta) prod_w (v_w + beta k_w zeta + gamma) - alpha perm prod_(w<4) (v_w + beta sigma_w + gamma)
+ * + alpha^2 L_1(zeta) (z(zeta) - 1), where r's third line is the terms with z(zeta) and the last factor (d + beta sigma_4 + gamma) splits
+ * into r's fourth line and -alpha perm (...)(...)(...)(d + gamma).  Hence
+ *   quot * Z_H(zeta) = lin + PI(zeta) - alpha^2 L_1(zeta) - alpha perm (a + beta sigma_1 + gamma)(b + beta sigma_2 + gamma)(c + beta sigma_3 + gamma)(d + gamma),
+ * which is what the verifier's compute_quotient_evaluation checks.  On a composer that violates a constraint it fails (t is then not
+ * the exact quotient), as the verifier would see.
+ * pg_prover_openings: evals (host) and dst = [W_zeta, W_zeta_w, r], 3 x N coefficients column-major.  It rebuilds the wire, z, sigma and
+ * selector coefficient vectors (as pg_quotient does) and takes t as input.  The remainder of each division is the aggregate's value at
+ * its point; the call compares it with the same sum formed from the evaluations and reports a mismatch as PG_ERR_CUDA.  It does not
+ * judge the witness.  PG_ERR_ARG: 2^log_n < the circuit size or log_n > 30, a null buffer, an unreduced challenge, an unreduced
+ * coefficient of t (counted on the device; pg_last_error names the first, as index r*N + m), zeta^N = 1 (zeta in H: the reference's
+ * L_1 inversion panics at zeta = 1 and the verifier divides by Z_H(zeta)), or a zero z denominator (pg_last_error names the row).
+ * PG_ERR_STATE on a ctx whose communicator has more than one rank.  It synchronises the ctx stream. */
+typedef struct pg_proof_evaluations {
+    pg_fr a_eval, b_eval, c_eval, d_eval, a_next_eval, b_next_eval, d_next_eval, q_arith_eval, q_c_eval, q_l_eval, q_r_eval,
+          left_sigma_eval, right_sigma_eval, out_sigma_eval, lin_poly_eval, perm_eval, quot_eval;
+} pg_proof_evaluations;
+int pg_prover_openings(pg_ctx *ctx, uint32_t log_n, const pg_fr *challenges, const pg_fr *t, int t_on_device, pg_proof_evaluations *evals,
+                       pg_fr *dst, int dst_on_device);
+
 /* ---- commitments (SURVEY.md section 8f item 2, second half) -----------------------------------------------------------------
  * KZG commitments of coefficient vectors in the BLS12-381 group G1 [DEP dusk-plonk 0.8 CommitKey::commit =
  * dusk-bls12_381 msm_variable_base(&powers_of_g, &poly.coeffs); Prover::prove computes w_l_poly_commit .. w_4_poly_commit right
@@ -445,7 +488,8 @@ int pg_microbench(pg_ctx *ctx, int mode, double *ops_per_s);
 
 /* Element-wise Fr self-test kernels (op: 0 mul, 1 add, 2 sub, 3 neg, 4 invert-or-zero (batch inversion), 5 from_mont,
  * 6 mul via the portable CIOS path, 7 exclusive prefix product out[0] = 1, out[i] = a[0]*..*a[i-1] (the grand-product scan of
- * pg_permutation_z)).  a, b, out: host arrays of n scalars. */
+ * pg_permutation_z), 8 division by (X - b[0]): out[0 .. n-1) = ruffini(a, b[0]) and out[n-1] = the remainder a(b[0]) (the Ruffini scan of
+ * pg_prover_openings; b holds one scalar)).  a, b, out: host arrays of n scalars. */
 int pg_fr_op(pg_ctx *ctx, int op, uint64_t n, const pg_fr *a, const pg_fr *b, pg_fr *out);
 
 #ifdef __cplusplus

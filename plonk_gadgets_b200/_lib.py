@@ -46,7 +46,7 @@ class pg_check_stats(C.Structure):
     _fields_ = [("launches", C.c_uint64 * 8), ("rows", C.c_uint64 * 8)]
 
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 # every symbol include/pg_b200.h declares: name -> (restype, argtypes)
 _vp, _u64, _i32, _u32 = C.c_void_p, C.c_uint64, C.c_int, C.c_uint32
@@ -98,6 +98,7 @@ SIGNATURES = {
     "pg_selector_polynomials": (_i32, [_vp, _u32, _i32, _vp, _i32]),
     "pg_public_input_polynomial": (_i32, [_vp, _u32, _i32, _vp, _i32]),
     "pg_quotient": (_i32, [_vp, _u32, _vp, _vp, _vp, _vp, _vp, _i32]),
+    "pg_prover_openings": (_i32, [_vp, _u32, _vp, _vp, _i32, _vp, _vp, _i32]),
     "pg_msm": (_i32, [_vp, _u64, _vp, _vp, _vp, _i32]),
     "pg_srs_powers": (_i32, [_vp, _vp, _vp, _u64, _vp, _i32]),
     "pg_g1_fixed_base_mul": (_i32, [_vp, _u64, _vp, _vp, _vp, _i32]),

@@ -30,6 +30,9 @@ CHECK_GENERIC, CHECK_SPARSE = 0, 1
 F_TIMING = 1
 F_FUSED_CHECK = 2
 FORM_EVALUATIONS, FORM_COEFFICIENTS = 0, 1
+# pg_proof_evaluations: dusk-plonk 0.8 ProofEvaluations' fields in order, then the quotient's evaluation at the challenge
+OPENING_EVALUATIONS = ("a_eval", "b_eval", "c_eval", "d_eval", "a_next_eval", "b_next_eval", "d_next_eval", "q_arith_eval", "q_c_eval",
+                       "q_l_eval", "q_r_eval", "left_sigma_eval", "right_sigma_eval", "out_sigma_eval", "lin_poly_eval", "perm_eval", "quot_eval")
 UINT64_MAX = 2 ** 64 - 1
 
 
@@ -482,6 +485,36 @@ class StandardComposer:
         dst = np.empty((4, 1 << log_n, 4), dtype=np.uint64)
         self._ok(self._L.pg_quotient(self._ctx, log_n, *map(vp, ch), vp(dst), 0), "pg_quotient")
         return dst
+
+    # -- openings: prover rounds 4 and 5 ([DEP] Prover::prove, linearisation_poly::compute, Polynomial::ruffini)
+    def prover_openings(self, t, alpha, beta, gamma, range_challenge, z, v, v_shifted, log_n: int | None = None, out=None):
+        """Prover rounds 4 and 5 for pg_quotient's t_1 .. t_4 (a (4, 2^log_n, 4) host array or device tensor) and the challenges (one
+        Montgomery scalar each; z is the evaluation challenge, v / v_shifted aggregate the openings at z and z*w): (evaluations, openings).
+        evaluations: dict name -> (4,) uint64 in ProofEvaluations' order plus quot_eval (OPENING_EVALUATIONS); openings: [W_z, W_zw, r],
+        (3, 2^log_n, 4) uint64 coefficients (or written to the device tensor `out`).  log_n <= 30."""
+        log_n = self._domain(log_n)
+        if log_n > 30:
+            raise EngineError(-2, "pg_prover_openings", f"log_n = {log_n}: the quotient's domain bound is 2^30")
+        ch = np.ascontiguousarray(np.stack([np.ascontiguousarray(x, dtype=np.uint64).reshape(4)
+                                            for x in (alpha, beta, gamma, range_challenge, z, v, v_shifted)]))
+        vp = lambda x: x.ctypes.data_as(C.c_void_p)
+        ev = np.zeros((len(OPENING_EVALUATIONS), 4), dtype=np.uint64)
+        if isinstance(t, np.ndarray):
+            t = np.ascontiguousarray(t, dtype=np.uint64)
+            if t.shape != (4, 1 << log_n, 4):
+                raise EngineError(-2, "pg_prover_openings", f"t has shape {t.shape}, expected {(4, 1 << log_n, 4)}")
+            t_ptr, t_dev = vp(t), 0
+        else:
+            if tuple(t.shape) != (4, 1 << log_n, 4) or not t.is_contiguous():
+                raise EngineError(-2, "pg_prover_openings", f"t must be a contiguous (4, 2^{log_n}, 4) tensor")
+            t_ptr, t_dev = C.c_void_p(t.data_ptr()), 1
+        if out is not None:
+            self._ok(self._L.pg_prover_openings(self._ctx, log_n, vp(ch), t_ptr, t_dev, vp(ev), C.c_void_p(out.data_ptr()), 1), "pg_prover_openings")
+            dst = out
+        else:
+            dst = np.empty((3, 1 << log_n, 4), dtype=np.uint64)
+            self._ok(self._L.pg_prover_openings(self._ctx, log_n, vp(ch), t_ptr, t_dev, vp(ev), vp(dst), 0), "pg_prover_openings")
+        return dict(zip(OPENING_EVALUATIONS, ev)), dst
 
     # -- commitments: G1 multi-scalar multiplication, SRS powers, wire-polynomial commitments ([DEP] dusk-plonk 0.8 / dusk-bls12_381)
     @staticmethod

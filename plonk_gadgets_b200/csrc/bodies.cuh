@@ -1105,6 +1105,77 @@ struct FillBody {
     PG_HD static void run(const Args& a, uint64_t i) { aos_store(a.data, i, a.v); }
 };
 
+// ---------------------------------------------------------------------------------------------------- openings (rounds 4 and 5)
+// [DEP] dusk-plonk 0.8 Prover::prove (evaluations, linearisation_poly::compute, compute_quotient_opening_poly /
+// compute_aggregate_witness), recalled.  Vectors: the QV_PI coefficient vectors of the quotient (wires, z, sigma, selectors; QV_*
+// order) and t_1 .. t_4 (OV_T ..).  Pairs (vector, point): every vector at zeta (pair = vector), and w_l, w_r, w_4, z at zeta*w
+// (OV_SHIFTED ..).
+enum : uint32_t { OV_T = QV_PI, OV_VEC = OV_T + 4, OV_SHIFTED = OV_VEC, OV_PAIRS = OV_SHIFTED + 4 };
+PG_HD int open_shift_slot(uint32_t v) { return v == QV_W ? 0 : v == QV_W + 1 ? 1 : v == QV_W + 3 ? 2 : v == QV_Z ? 3 : -1; }
+// Evaluation pass, index i = v * s + j (j < s, s | len = N): partial[pair][j] = p^j * sum_k c_v[j + k s] (p^s)^k by Horner over the strided
+// coefficients, for p = zeta and, for the shifted vectors, zeta*w.  One Fr multiplication per coefficient and pair.  The t vectors
+// are caller input: an unreduced coefficient is counted in CNT_UNSAT / CNT_FIRST_BAD (index r * n + m of t).
+struct OpenEvalBody {
+    struct Args { const uint4* coef; const uint4* t; uint64_t len, s, n /* OV_VEC * s */; uint32_t log_lo; const uint4* tab[2]; Fr step[2];
+                  uint4* partial; unsigned long long* counters; };
+    PG_HD static void run(const Args& a, uint64_t i) {
+        const uint32_t v = (uint32_t)(i / a.s); const uint64_t j = i % a.s;
+        const uint4* c = v < OV_T ? a.coef + 2 * (uint64_t)v * a.len : a.t + 2 * (uint64_t)(v - OV_T) * a.len;
+        const int sh = open_shift_slot(v);
+        Fr acc = fr_zero(), acc2 = fr_zero();
+        for (uint64_t m = a.len - a.s + j;; m -= a.s) {
+            const Fr x = aos_load(c, m);
+            if (v >= OV_T && !fr_is_reduced(x)) { counter_add(a.counters + CNT_UNSAT, 1ull); counter_min(a.counters + CNT_FIRST_BAD, (unsigned long long)((v - OV_T) * a.len + m)); }
+            acc = fr_add(fr_mul(acc, a.step[0]), x);
+            if (sh >= 0) acc2 = fr_add(fr_mul(acc2, a.step[1]), x);
+            if (m < a.s) break;
+        }
+        aos_store(a.partial, (uint64_t)v * a.s + j, fr_mul(acc, pow_table_at(a.tab[0], a.log_lo, j)));
+        if (sh >= 0) aos_store(a.partial, (uint64_t)(OV_SHIFTED + sh) * a.s + j, fr_mul(acc2, pow_table_at(a.tab[1], a.log_lo, j)));
+    }
+};
+// out[i] = sum_(k < len) in[i * len + k], i < n
+struct OpenSumBody {
+    struct Args { const uint4* in; uint4* out; uint64_t len, n; };
+    PG_HD static void run(const Args& a, uint64_t i) {
+        Fr s = fr_zero();
+        for (uint64_t k = 0; k < a.len; k++) s = fr_add(s, aos_load(a.in, i * a.len + k));
+        aos_store(a.out, i, s);
+    }
+};
+// Combination pass, pointwise over the coefficients m: out = [agg_zeta, agg_zeta_w, r] (3 x n), with the host's weights
+//   r          = rw . (q_m, q_l, q_r, q_o, q_4, q_c, q_range, z, sigma_4)
+//   agg_zeta   = t_1 + zeta^N t_2 + zeta^2N t_3 + zeta^3N t_4 + v r + v^2 w_l + v^3 w_r + v^4 w_o + v^5 w_4 + v^6 sigma_1 + v^7 sigma_2 + v^8 sigma_3
+//   agg_zeta_w = z + v' w_l + v'^2 w_r + v'^3 w_4
+// 23 Montgomery multiplications per coefficient.
+struct OpenCombineBody {
+    struct Args { const uint4* coef; const uint4* t; uint64_t n; Fr rw[9]; Fr zn[3]; Fr v[8]; Fr vs[3]; uint4* out; };
+    PG_HD static Fr ld(const Args& a, uint32_t v, uint64_t m) { return aos_load(a.coef, (uint64_t)v * a.n + m); }
+    PG_HD static void run(const Args& a, uint64_t m) {
+        Fr r = fr_mul(a.rw[0], ld(a, QV_QM, m));
+#pragma unroll
+        for (int k = 1; k < 6; k++) r = fr_add(r, fr_mul(a.rw[k], ld(a, QV_QM + k, m)));      // q_l q_r q_o q_4 q_c
+        r = fr_add(r, fr_mul(a.rw[6], ld(a, QV_QRANGE, m)));
+        r = fr_add(r, fr_mul(a.rw[7], ld(a, QV_Z, m)));
+        r = fr_add(r, fr_mul(a.rw[8], ld(a, QV_S + 3, m)));
+        Fr g = aos_load(a.t, m);
+#pragma unroll
+        for (int k = 0; k < 3; k++) g = fr_add(g, fr_mul(a.zn[k], aos_load(a.t, (uint64_t)(k + 1) * a.n + m)));
+        g = fr_add(g, fr_mul(a.v[0], r));
+#pragma unroll
+        for (int k = 0; k < 4; k++) g = fr_add(g, fr_mul(a.v[1 + k], ld(a, QV_W + k, m)));
+#pragma unroll
+        for (int k = 0; k < 3; k++) g = fr_add(g, fr_mul(a.v[5 + k], ld(a, QV_S + k, m)));
+        Fr h = ld(a, QV_Z, m);
+        h = fr_add(h, fr_mul(a.vs[0], ld(a, QV_W, m)));
+        h = fr_add(h, fr_mul(a.vs[1], ld(a, QV_W + 1, m)));
+        h = fr_add(h, fr_mul(a.vs[2], ld(a, QV_W + 3, m)));
+        aos_store(a.out, m, g);
+        aos_store(a.out, a.n + m, h);
+        aos_store(a.out, 2 * a.n + m, r);
+    }
+};
+
 // ---------------------------------------------------------------------------------------------------- synthetic inputs
 PG_HD uint64_t splitmix64_at(uint64_t seed, uint64_t index1) {   // output number index1 (1-based) of SplitMix64(seed)
     uint64_t z = seed + index1 * 0x9E3779B97F4A7C15ull;

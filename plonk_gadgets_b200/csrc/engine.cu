@@ -447,6 +447,27 @@ public:
         k_fr_scan_apply<<<(unsigned)tiles, SCAN_THREADS, 0, stream>>>(in, out, n, scratch, nullptr);
         return launched("k_fr_scan_apply");
     }
+    // Ruffini division (scan.cuh) of n scalars by (X - p): out[i] = s_(i+1), *rem = f(p); pw: fr_ruffini_levels(n) tables of RUF_TAB
+    // powers (level l: of p^(SCAN_TILE^l)); scratch: fr_scan_scratch(n) scalars
+    bool run_fr_ruffini(const uint4* in, uint4* out, uint64_t n, const uint4* pw, uint4* rem, uint4* scratch) {
+        if (!n) return true;
+        tic(CLS_OTHER, 0);
+        const bool ok = fr_ruffini_level(in, out, n, pw, rem, scratch);
+        toc();
+        return ok;
+    }
+    bool fr_ruffini_level(const uint4* in, uint4* out, uint64_t n, const uint4* pw, uint4* rem, uint4* scratch) {
+        if (n <= SCAN_TILE) {
+            k_fr_ruffini_apply<<<1, SCAN_THREADS, 0, stream>>>(in, out, n, pw, nullptr, rem);
+            return launched("k_fr_ruffini_apply");
+        }
+        const uint64_t tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
+        k_fr_ruffini_reduce<<<(unsigned)tiles, SCAN_THREADS, 0, stream>>>(in, n, pw, scratch);
+        if (!launched("k_fr_ruffini_reduce")) return false;
+        if (!fr_ruffini_level(scratch, scratch, tiles, pw + 2 * RUF_TAB, rem, scratch + 2 * tiles)) return false;   // tile values -> their carries
+        k_fr_ruffini_apply<<<(unsigned)tiles, SCAN_THREADS, 0, stream>>>(in, out, n, pw, scratch, nullptr);
+        return launched("k_fr_ruffini_apply");
+    }
     bool run_check_rows(const CheckRowsBody::Args& a) {
         tic(CLS_CHECK, a.n);
         k_check_rows<<<grid_for(a.n), BLOCK, 0, stream>>>(a);
@@ -528,6 +549,7 @@ public:
 };
 
 static_assert(has_fr_scan<CudaBackend>::value, "the shipped library computes the grand product with the device-wide scan of scan.cuh");
+static_assert(has_fr_ruffini<CudaBackend>::value, "the shipped library divides the opening aggregates with the device-wide Ruffini scan of scan.cuh");
 
 }  // namespace pg
 

@@ -20,6 +20,8 @@
 //   bool run_ntt_pass(const NttPassArgs&, uint64_t n_blocks)    -- one group of butterfly stages over all tiles (ntt.cuh)
 //   bool run_fr_scan(const uint4* in, uint4* out, uint64_t n, uint4* total, uint4* scratch) -- exclusive prefix product (scan.cuh);
 //        optional: a backend without it (the test-only loop backend) runs FrScanSerialBody, the defining serial loop
+//   bool run_fr_ruffini(const uint4* in, uint4* out, uint64_t n, const uint4* pw, uint4* rem, uint4* scratch) -- division by (X - p)
+//        (scan.cuh); optional like run_fr_scan: without it FrRuffiniSerialBody runs
 //   bool upload_pow2(const Fr*), bool imad_peak(double*, double*), bool ubench(int, double*), timing(pg_timing*, bool reset)
 #pragma once
 #include <stdio.h>
@@ -88,9 +90,19 @@ inline Fr fr_from_pg(const pg_fr& x) {
     return r;
 }
 
+static_assert(sizeof(pg_proof_evaluations) == 17 * sizeof(pg_fr), "pg_proof_evaluations is 17 consecutive scalars");
+inline pg_fr fr_to_pg(const Fr& x) {
+    pg_fr r;
+    for (int i = 0; i < 4; i++) r.l[i] = (uint64_t)x.v[2 * i] | ((uint64_t)x.v[2 * i + 1] << 32);
+    return r;
+}
+
 // whether a backend brings its own device-wide prefix product (Engine::fr_scan)
 template <class B, class = void> struct has_fr_scan : std::false_type {};
 template <class B> struct has_fr_scan<B, std::void_t<decltype(&B::run_fr_scan)>> : std::true_type {};
+// whether a backend brings its own device-wide Ruffini division (Engine::fr_ruffini)
+template <class B, class = void> struct has_fr_ruffini : std::false_type {};
+template <class B> struct has_fr_ruffini<B, std::void_t<decltype(&B::run_fr_ruffini)>> : std::true_type {};
 
 template <class BE>
 class Engine {
@@ -1465,6 +1477,19 @@ public:
         release_scratch_from(mark);
         return rc;
     }
+    // The coefficient vectors of rounds 3 to 5, 2^log_n each in QV_* order: wires, z (for beta, gamma), sigma, the eight selectors and,
+    // with_pi, PI (coef holds QV_COEF vectors then, else QV_PI)
+    int component_polynomials(uint32_t log_n, const pg_fr* beta, const pg_fr* gamma, bool with_pi, uint4* coef) {
+        const uint64_t n = 1ull << log_n;
+        auto col = [n, coef](uint32_t v) { return (pg_fr*)(coef + 2 * (uint64_t)v * n); };
+        int rc;
+        if ((rc = wire_polynomials(log_n, col(QV_W), 1))) return rc;
+        if ((rc = permutation_z(log_n, beta, gamma, PG_FORM_COEFFICIENTS, col(QV_Z), 1, nullptr))) return rc;
+        if ((rc = sigma_polynomials(log_n, PG_FORM_COEFFICIENTS, col(QV_S), 1))) return rc;
+        if ((rc = selector_polynomials(log_n, PG_FORM_COEFFICIENTS, col(QV_QM), 1))) return rc;
+        if (with_pi && (rc = public_input_polynomial(log_n, PG_FORM_COEFFICIENTS, col(QV_PI), 1))) return rc;
+        return PG_OK;
+    }
     static Fr fr_small(uint64_t v) { Fr raw = fr_zero(); raw.v[0] = (uint32_t)v; raw.v[1] = (uint32_t)(v >> 32); return fr_to_mont(raw); }
     static Fr fr_pow2k(Fr x, uint32_t k) { for (uint32_t i = 0; i < k; i++) x = fr_sqr(x); return x; }     // x^(2^k)
     // Round 3: t_1 .. t_4 (4 columns of N = 2^log_n coefficients).  Coefficient vectors of the wires, z, sigma, the selectors and PI
@@ -1489,11 +1514,7 @@ public:
         auto col = [n](uint4* base, uint32_t v) { return base + 2 * (uint64_t)v * n; };
         uint4* coef = (uint4*)dalloc(QV_COEF * n * sizeof(pg_fr)); if (!coef) return fail(PG_ERR_OOM, "quotient coefficient vectors");
         scratch.push_back(coef);
-        if ((rc = wire_polynomials(log_n, (pg_fr*)col(coef, QV_W), 1))) return rc;
-        if ((rc = permutation_z(log_n, beta, gamma, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_Z), 1, nullptr))) return rc;
-        if ((rc = sigma_polynomials(log_n, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_S), 1))) return rc;
-        if ((rc = selector_polynomials(log_n, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_QM), 1))) return rc;
-        if (has_pi && (rc = public_input_polynomial(log_n, PG_FORM_COEFFICIENTS, (pg_fr*)col(coef, QV_PI), 1))) return rc;
+        if ((rc = component_polynomials(log_n, beta, gamma, has_pi, coef))) return rc;
         uint4* ev = (uint4*)dalloc(QV_EV * n * sizeof(pg_fr)); if (!ev) return fail(PG_ERR_OOM, "quotient evaluation vectors");
         scratch.push_back(ev);
         uint4* out = reinterpret_cast<uint4*>(dst);
@@ -1545,6 +1566,143 @@ public:
         if (!be.template run_simple<QuotientSplitBody>(s, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "quotient split kernel");
         if (!dst_on_device) { if ((rc = deliver(dst, out, 4 * n * sizeof(pg_fr), 0))) return rc; }
         else if (!be.sync()) return fail(PG_ERR_CUDA, "sync");                            // the coefficient and evaluation vectors go back to the pool
+        release_scratch_from(mark);
+        return PG_OK;
+    }
+
+    // ------------------------------------------------------------------------------------------------ openings (rounds 4 and 5)
+    // [DEP dusk-plonk 0.8 Prover::prove, linearisation_poly::compute, compute_quotient_opening_poly / compute_aggregate_witness,
+    // Polynomial::ruffini, recalled]; bodies.cuh OpenEvalBody / OpenSumBody / OpenCombineBody, scan.cuh (Ruffini division).
+    // out[i] = s_(i+1) of s_i = f_i + p s_(i+1) and *rem = f(p) (in place allowed): the backend's device-wide scan (CudaBackend::
+    // run_fr_ruffini; engine.cu asserts that it has one), else FrRuffiniSerialBody as one unit of work
+    int fr_ruffini(const uint4* in, uint4* out, uint64_t n, const Fr& p, uint4* rem) {
+        if constexpr (has_fr_ruffini<BE>::value) {
+            const uint32_t levels = fr_ruffini_levels(n);
+            std::vector<Fr> host(levels * RUF_TAB);
+            Fr x = p;                                                       // level l: powers of p^(SCAN_TILE^l)
+            for (uint32_t l = 0; l < levels; l++) {
+                Fr y = fr_one();
+                for (uint64_t k = 0; k < RUF_TAB; k++) { host[l * RUF_TAB + k] = y; y = fr_mul(y, x); }
+                x = host[l * RUF_TAB + SCAN_TILE];
+            }
+            uint4* pw = (uint4*)dalloc((host.size() + fr_scan_scratch(n)) * sizeof(pg_fr)); if (!pw) return fail(PG_ERR_OOM, "ruffini tables");
+            scratch.push_back(pw);
+            if (!be.h2d(pw, host.data(), host.size() * sizeof(pg_fr))) return fail(PG_ERR_CUDA, "ruffini table copy");
+            if (!be.run_fr_ruffini(in, out, n, pw, rem, pw + 2 * host.size())) return fail(PG_ERR_CUDA, "ruffini scan");
+        } else {
+            const FrRuffiniSerialBody::Args a{in, out, n, p, rem};
+            if (!be.template run_simple<FrRuffiniSerialBody>(a, 1, CLS_OTHER)) return fail(PG_ERR_CUDA, "ruffini loop");
+        }
+        return PG_OK;
+    }
+    // Rounds 4 and 5 for the caller's challenges (alpha beta gamma rho zeta v v') and t = pg_quotient's t_1 .. t_4: the 17 evaluations
+    // (pg_proof_evaluations), and dst = [W_zeta, W_zeta_w, r] (3 x 2^log_n coefficients).  Coefficient vectors as for the quotient,
+    // one evaluation pass over them (25 pairs), the weights on the host, one combination pass, two in-place Ruffini divisions whose
+    // remainders must equal the aggregates' values computed from the evaluations.
+    int prover_openings(uint32_t log_n, const pg_fr* challenges, const pg_fr* t_in, int t_on_device, pg_proof_evaluations* evals, pg_fr* dst,
+                        int dst_on_device) {
+        int rc;
+        if ((rc = perm_unsharded("prover_openings"))) return rc;
+        if (log_n > NTT_TWO_ADICITY - 2 || (1ull << log_n) < n_rows)
+            return fail(PG_ERR_ARG, "prover_openings: domain smaller than the circuit, or larger than 2^30 (pg_quotient's bound)");
+        if (!challenges || !t_in || !evals || !dst) return fail(PG_ERR_ARG, "prover_openings: null argument");
+        for (int k = 0; k < 7; k++)
+            if (!host_reduced(challenges[k])) return fail(PG_ERR_ARG, "prover_openings: a challenge (alpha beta gamma rho zeta v v') not fully reduced (>= q)");
+        const uint64_t n = 1ull << log_n;
+        const Fr al = fr_from_pg(challenges[0]), bt = fr_from_pg(challenges[1]), ga = fr_from_pg(challenges[2]), rh = fr_from_pg(challenges[3]);
+        const Fr zt = fr_from_pg(challenges[4]), v = fr_from_pg(challenges[5]), vs = fr_from_pg(challenges[6]);
+        const Fr one = fr_one(), zt_n = fr_pow2k(zt, log_n);
+        if (fr_eq(zt_n, one)) return fail(PG_ERR_ARG, "prover_openings: zeta^N = 1 (zeta in the domain: L_1(zeta) and the verifier's 1 / Z_H(zeta) do not exist)");
+        const Fr omega = fr_pow2k(fr_root_of_unity(), NTT_TWO_ADICITY - log_n), zw = fr_mul(zt, omega);
+        const size_t mark = scratch.size();
+        const uint4* t = stage(t_in, 4 * n, t_on_device, &rc); if (!t) return rc;
+        uint4* coef = (uint4*)dalloc(QV_PI * n * sizeof(pg_fr)); if (!coef) return fail(PG_ERR_OOM, "opening coefficient vectors");
+        scratch.push_back(coef);
+        if ((rc = component_polynomials(log_n, &challenges[1], &challenges[2], false, coef))) return rc;
+        // evaluation pass: s strided Horner chains per vector, partial sums of 2^7 then the rest
+        const uint32_t log_s = std::min<uint32_t>(log_n, 14), log_g = std::min<uint32_t>(log_s, 7);
+        const uint64_t s = 1ull << log_s, g = 1ull << log_g;
+        const uint64_t entries = pow_table_entries(log_s);
+        std::vector<Fr> host_tabs(2 * entries);
+        pow_table_host(zt, log_s, host_tabs.data());
+        pow_table_host(zw, log_s, host_tabs.data() + entries);
+        uint4* buf = (uint4*)dalloc((host_tabs.size() + OV_PAIRS * s + OV_PAIRS * (s / g) + 2) * sizeof(pg_fr));
+        if (!buf) return fail(PG_ERR_OOM, "evaluation buffers");
+        scratch.push_back(buf);
+        uint4* partial = buf + 2 * host_tabs.size(); uint4* partial2 = partial + 2 * OV_PAIRS * s; uint4* rem = partial2 + 2 * OV_PAIRS * (s / g);
+        if (!be.h2d(buf, host_tabs.data(), host_tabs.size() * sizeof(pg_fr))) return fail(PG_ERR_CUDA, "power table copy");
+        if ((rc = reset_counters())) return rc;
+        OpenEvalBody::Args ea; memset(&ea, 0, sizeof(ea));
+        ea.coef = coef; ea.t = t; ea.len = n; ea.s = s; ea.n = OV_VEC * s; ea.log_lo = pow_table_log_lo(log_s); ea.tab[0] = buf; ea.tab[1] = buf + 2 * entries;
+        ea.step[0] = fr_pow2k(zt, log_s); ea.step[1] = fr_pow2k(zw, log_s); ea.partial = partial; ea.counters = d_counters;
+        if (!be.template run_simple<OpenEvalBody>(ea, OV_VEC * s, CLS_OTHER)) return fail(PG_ERR_CUDA, "evaluation kernel");
+        OpenSumBody::Args s1{partial, partial2, g, OV_PAIRS * (s / g)}, s2{partial2, partial, s / g, OV_PAIRS};
+        if (!be.template run_simple<OpenSumBody>(s1, OV_PAIRS * (s / g), CLS_OTHER) || !be.template run_simple<OpenSumBody>(s2, OV_PAIRS, CLS_OTHER))
+            return fail(PG_ERR_CUDA, "evaluation sum kernel");
+        unsigned long long c[CNT_WORDS];
+        if ((rc = read_counters(c))) return rc;
+        if (c[CNT_UNSAT]) {
+            char msg[200];
+            snprintf(msg, sizeof(msg), "prover_openings: %llu coefficient(s) of t not fully reduced (>= q), first at index %llu", c[CNT_UNSAT], c[CNT_FIRST_BAD]);
+            return fail(PG_ERR_ARG, msg);
+        }
+        pg_fr ev_pg[OV_PAIRS];
+        if ((rc = deliver(ev_pg, partial, sizeof(ev_pg), 0))) return rc;
+        Fr e[OV_PAIRS];
+        for (uint32_t k = 0; k < OV_PAIRS; k++) e[k] = fr_from_pg(ev_pg[k]);
+        const Fr a_ = e[QV_W], b_ = e[QV_W + 1], c_ = e[QV_W + 2], d_ = e[QV_W + 3], aw = e[OV_SHIFTED], bw = e[OV_SHIFTED + 1], dw = e[OV_SHIFTED + 2];
+        const Fr zw_ = e[OV_SHIFTED + 3];
+        const Fr zt_2n = fr_mul(zt_n, zt_n), zt_3n = fr_mul(zt_2n, zt_n);
+        const Fr t_bar = fr_add(fr_add(e[OV_T], fr_mul(zt_n, e[OV_T + 1])), fr_add(fr_mul(zt_2n, e[OV_T + 2]), fr_mul(zt_3n, e[OV_T + 3])));
+        // linearisation weights: r = rw . (q_m q_l q_r q_o q_4 q_c q_range z sigma_4)
+        const Fr qa = e[QV_QARITH], two = fr_small(2), three = fr_small(3), kappa = fr_sqr(rh);
+        Fr rw[9];
+        rw[0] = fr_mul(qa, fr_mul(a_, b_)); rw[1] = fr_mul(qa, a_); rw[2] = fr_mul(qa, b_); rw[3] = fr_mul(qa, c_); rw[4] = fr_mul(qa, d_); rw[5] = qa;
+        Fr rng = quot_delta(fr_sub(dw, quot_times4(a_)), two, three);
+        rng = fr_add(fr_mul(rng, kappa), quot_delta(fr_sub(a_, quot_times4(b_)), two, three));
+        rng = fr_add(fr_mul(rng, kappa), quot_delta(fr_sub(b_, quot_times4(c_)), two, three));
+        rng = fr_add(fr_mul(rng, kappa), quot_delta(fr_sub(c_, quot_times4(d_)), two, three));
+        rw[6] = fr_mul(rh, rng);
+        const Fr wv[4] = {a_, b_, c_, d_};
+        Fr prod_id = one, prod_sig = one;                                   // prod_w (v_w + beta k_w zeta + gamma), prod_(w<3) (v_w + beta sigma_w + gamma)
+        for (uint32_t w = 0; w < 4; w++) {
+            prod_id = fr_mul(prod_id, fr_add(fr_add(wv[w], fr_mul(fr_mul(bt, perm_coset(w)), zt)), ga));
+            if (w < 3) prod_sig = fr_mul(prod_sig, fr_add(fr_add(wv[w], fr_mul(bt, e[QV_S + w])), ga));
+        }
+        const Fr alpha2 = fr_sqr(al);
+        const Fr l1 = fr_mul(fr_sub(zt_n, one), fr_inv_fermat(fr_mul(fr_small(n), fr_sub(zt, one))));       // (zeta^N - 1) / (N (zeta - 1))
+        rw[7] = fr_add(fr_mul(al, prod_id), fr_mul(alpha2, l1));
+        rw[8] = fr_neg(fr_mul(fr_mul(fr_mul(al, bt), zw_), prod_sig));
+        const uint32_t r_terms[9] = {QV_QM, QV_QL, QV_QR, QV_QO, QV_Q4, QV_QC, QV_QRANGE, QV_Z, QV_S + 3};
+        Fr r_bar = fr_zero();
+        for (int k = 0; k < 9; k++) r_bar = fr_add(r_bar, fr_mul(rw[k], e[r_terms[k]]));
+        const Fr out_ev[17] = {a_, b_, c_, d_, aw, bw, dw, qa, e[QV_QC], e[QV_QL], e[QV_QR], e[QV_S], e[QV_S + 1], e[QV_S + 2], r_bar, zw_, t_bar};
+        // combination pass
+        uint4* out = reinterpret_cast<uint4*>(dst);
+        if (!dst_on_device) { out = (uint4*)dalloc(3 * n * sizeof(pg_fr)); if (!out) return fail(PG_ERR_OOM, "opening buffer"); scratch.push_back(out); }
+        OpenCombineBody::Args ca; memset(&ca, 0, sizeof(ca));
+        ca.coef = coef; ca.t = t; ca.n = n; ca.out = out;
+        for (int k = 0; k < 9; k++) ca.rw[k] = rw[k];
+        ca.zn[0] = zt_n; ca.zn[1] = zt_2n; ca.zn[2] = zt_3n;
+        ca.v[0] = v; for (int k = 1; k < 8; k++) ca.v[k] = fr_mul(ca.v[k - 1], v);
+        ca.vs[0] = vs; ca.vs[1] = fr_mul(vs, vs); ca.vs[2] = fr_mul(ca.vs[1], vs);
+        if (!be.template run_simple<OpenCombineBody>(ca, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "combination kernel");
+        // the aggregates' values at their points, from the evaluations
+        const Fr agg_at[2] = {
+            [&] { Fr x = t_bar; const Fr p[8] = {r_bar, a_, b_, c_, d_, e[QV_S], e[QV_S + 1], e[QV_S + 2]};
+                  for (int k = 0; k < 8; k++) x = fr_add(x, fr_mul(ca.v[k], p[k])); return x; }(),
+            fr_add(fr_add(zw_, fr_mul(ca.vs[0], aw)), fr_add(fr_mul(ca.vs[1], bw), fr_mul(ca.vs[2], dw)))};
+        const Fr pts[2] = {zt, zw};
+        for (int k = 0; k < 2; k++)
+            if ((rc = fr_ruffini(out + 2 * (uint64_t)k * n, out + 2 * (uint64_t)k * n, n, pts[k], rem + 2 * k))) return rc;
+        pg_fr rem_pg[2];
+        if ((rc = deliver(rem_pg, rem, sizeof(rem_pg), 0))) return rc;
+        for (int k = 0; k < 2; k++)
+            if (!fr_eq(fr_from_pg(rem_pg[k]), agg_at[k]))
+                return fail(PG_ERR_CUDA, k ? "prover_openings: the division's remainder differs from the zeta*w aggregate's evaluation"
+                                           : "prover_openings: the division's remainder differs from the zeta aggregate's evaluation");
+        for (int k = 0; k < 17; k++) reinterpret_cast<pg_fr*>(evals)[k] = fr_to_pg(out_ev[k]);      // the struct's 17 fields, in order
+        if (!dst_on_device && (rc = deliver(dst, out, 3 * n * sizeof(pg_fr), 0))) return rc;
         release_scratch_from(mark);
         return PG_OK;
     }
@@ -1657,7 +1815,8 @@ public:
         if (!a || !out) return fail(PG_ERR_ARG, "fr_op: null argument");
         const size_t mark = scratch.size();
         int rc; const uint4* da = stage(a, n, 0, &rc); if (!da) return rc;
-        const uint4* db = nullptr; if (b) { db = stage(b, n, 0, &rc); if (!db) return rc; }
+        if (op == 8 && !b) return fail(PG_ERR_ARG, "fr_op 8: null b");
+        const uint4* db = nullptr; if (b && op != 8) { db = stage(b, n, 0, &rc); if (!db) return rc; }
         uint4* dout = (uint4*)dalloc(n * sizeof(pg_fr)); if (!dout) return fail(PG_ERR_OOM, "fr_op buffer");
         scratch.push_back(dout);
         bool ok;
@@ -1670,6 +1829,15 @@ public:
             DevTab view; memset(&view, 0, sizeof(view)); view.fr = tab; view.stride = n;
             ColReadBody::Args rd{view, loc_make(LOC_FR, 0, 1), dout, n};
             ok = be.template run_simple<AddInputBody>(in, n, CLS_OTHER) && be.run_batch_inv(inv, CLS_OTHER) && be.template run_simple<ColReadBody>(rd, n, CLS_OTHER);
+        }
+        else if (op == 8) {  // Ruffini division by (X - b[0]) in place on the staged copy of a, the remainder a(b[0]) into out[n-1]
+            if (!host_reduced(*b)) return fail(PG_ERR_ARG, "fr_op 8: b[0] not fully reduced (>= q)");
+            uint4* rem = (uint4*)dalloc(sizeof(pg_fr)); if (!rem) return fail(PG_ERR_OOM, "fr_op remainder");
+            scratch.push_back(rem);
+            uint4* d = const_cast<uint4*>(da);
+            if ((rc = fr_ruffini(d, d, n, fr_from_pg(*b), rem))) return rc;
+            ok = be.d2d(d + 2 * (n - 1), rem, sizeof(pg_fr));
+            dout = d;
         }
         else if (op == 7) {  // exclusive prefix product through the grand-product scan (scan.cuh)
             uint4* tot = (uint4*)dalloc((1 + fr_scan_scratch(n)) * sizeof(pg_fr)); if (!tot) return fail(PG_ERR_OOM, "fr_op scan scratch");

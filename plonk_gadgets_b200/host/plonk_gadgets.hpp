@@ -191,6 +191,16 @@ public:
         ok(pg_quotient(ctx_, log_n, p(alpha), p(beta), p(gamma), p(range_challenge), reinterpret_cast<pg_fr*>(out.data()), 0), "pg_quotient");
         return out;
     }
+    /// prover rounds 4 and 5 for pg_quotient's t (4 x 2^log_n) and the challenges alpha beta gamma rho zeta v v': the 17 evaluations
+    /// (ProofEvaluations' order, then quot_eval) and [W_zeta, W_zeta_w, r], 3 x 2^log_n coefficients
+    std::pair<pg_proof_evaluations, std::vector<BlsScalar>> prover_openings(uint32_t log_n, const std::vector<BlsScalar>& t, const BlsScalar (&challenges)[7]) {
+        if (t.size() != ((size_t)4 << log_n)) throw std::invalid_argument("prover_openings: t must hold 4 x 2^log_n scalars");
+        pg_proof_evaluations ev;
+        std::vector<BlsScalar> out((size_t)3 << log_n);
+        ok(pg_prover_openings(ctx_, log_n, reinterpret_cast<const pg_fr*>(challenges), reinterpret_cast<const pg_fr*>(t.data()), 0, &ev,
+                              reinterpret_cast<pg_fr*>(out.data()), 0), "pg_prover_openings");
+        return {ev, out};
+    }
     /// EvaluationDomain::fft / ifft of 2^k scalars
     std::vector<BlsScalar> fft(const std::vector<BlsScalar>& v, bool inverse) {
         uint32_t log_n = 0; while ((1ull << log_n) < v.size()) log_n++;
