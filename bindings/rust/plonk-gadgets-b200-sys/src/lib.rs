@@ -181,6 +181,8 @@ extern "C" {
     pub fn pg_commit_wire_polynomials(ctx: *mut pg_ctx, log_n: u32, powers_of_g: *const pg_g1_affine, n_powers: u64, powers_on_device: c_int,
                                       out4: *mut pg_g1_affine) -> c_int;
     pub fn pg_srs_lagrange(ctx: *mut pg_ctx, beta: *const pg_fr, base: *const pg_g1_affine, log_n: u32, out: *mut pg_g1_affine, out_on_device: c_int) -> c_int;
+    pub fn pg_srs_lagrange_from_powers(ctx: *mut pg_ctx, log_n: u32, powers_of_g: *const pg_g1_affine, n_powers: u64, powers_on_device: c_int,
+                                       out: *mut pg_g1_affine, out_on_device: c_int) -> c_int;
     pub fn pg_commit_wire_evaluations(ctx: *mut pg_ctx, log_n: u32, lagrange: *const pg_g1_affine, n_points: u64, points_on_device: c_int,
                                       out4: *mut pg_g1_affine) -> c_int;
     pub fn pg_g1_op(ctx: *mut pg_ctx, op: c_int, n: u64, a: *const pg_g1_affine, b: *const pg_g1_affine, out: *mut pg_g1_affine) -> c_int;

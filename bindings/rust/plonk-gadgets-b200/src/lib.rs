@@ -259,6 +259,16 @@ impl BatchComposer {
         self.ok(unsafe { sys::pg_commit_wire_polynomials(self.ctx, log_n, powers_of_g.as_ptr(), powers_of_g.len() as u64, 0, out.as_mut_ptr()) })?;
         Ok(out)
     }
+    /// The Lagrange-basis form of the SRS for the domain 2^log_n from the CommitKey's monomial powers alone (beta unknown):
+    /// `out[i] = (1/n) sum_j w^(-ij) powers_of_g[j]` over the first n = 2^log_n powers, by an inverse FFT over G1 on the GPU.
+    pub fn srs_lagrange_from_powers(&mut self, log_n: u32, powers_of_g: &[sys::pg_g1_affine]) -> Result<Vec<sys::pg_g1_affine>, EngineError> {
+        let n = if log_n <= 32 { 1usize << log_n } else { 0 };           // log_n > 32: the call returns PG_ERR_ARG
+        let mut out = vec![sys::pg_g1_affine::default(); n];
+        self.ok(unsafe {
+            sys::pg_srs_lagrange_from_powers(self.ctx, log_n, powers_of_g.as_ptr(), powers_of_g.len() as u64, 0, out.as_mut_ptr(), 0)
+        })?;
+        Ok(out)
+    }
     /// The same four commitments from the wire values against the Lagrange-basis form of the SRS (`lagrange[i] = L_i(beta) * g`,
     /// exactly 2^log_n points): no FFT, and bits / short accumulators leave most windows of the multi-scalar multiplication empty.
     pub fn commit_wire_evaluations(&mut self, log_n: u32, lagrange: &[sys::pg_g1_affine]) -> Result<[sys::pg_g1_affine; 4], EngineError> {

@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define PG_B200_ABI_VERSION 6
+#define PG_B200_ABI_VERSION 7
 
 /* BlsScalar: ref:src/allocated_scalar.rs:9-12 (dusk_plonk::bls12_381::BlsScalar) */
 typedef struct pg_fr { uint64_t l[4]; } pg_fr;
@@ -430,9 +430,18 @@ int pg_commit_wire_polynomials(pg_ctx *ctx, uint32_t log_n, const pg_g1_affine *
  * commitment of a polynomial is sum_i f(w^i) * lagrange[i] -- the same group element as sum_j coeff_j * powers_of_g[j] -- so the
  * wire commitments can be taken from the wire VALUES directly: no FFT, and bits / short accumulators leave most windows empty.
  * pg_srs_lagrange builds that form for local setups that know beta (like PublicParameters::setup; PG_ERR_ARG if beta lies on the
- * domain); deriving it from monomial powers alone needs a group FFT (not built).  pg_commit_wire_evaluations returns the same four
- * points as pg_commit_wire_polynomials; n_points must be exactly 2^log_n. */
+ * domain).  pg_srs_lagrange_from_powers derives it from the monomial powers alone, for a trusted setup whose beta nobody knows.
+ * pg_commit_wire_evaluations returns the same four points as pg_commit_wire_polynomials; n_points must be exactly 2^log_n. */
 int pg_srs_lagrange(pg_ctx *ctx, const pg_fr *beta, const pg_g1_affine *base, uint32_t log_n, pg_g1_affine *out, int out_on_device);
+/* pg_srs_lagrange_from_powers: out[i] = (1/n) sum_{j<n} w^(-ij) * powers_of_g[j], i < n = 2^log_n, w the domain generator of pg_fft
+ * (EvaluationDomain::group_gen).  Only the first n powers are read (like the trimmed CommitKey).  When powers_of_g[j] = beta^j * base
+ * the result is pg_srs_lagrange(beta, base, log_n) bit for bit (canonical affine limbs, infinity all-zero).  log_n = 0 copies
+ * powers_of_g[0].  The work is an inverse FFT over G1 with a 255-bit scalar multiplication per butterfly (about
+ * (n/2) log n + n of them); it needs n x 192 bytes of device scratch.  Points are taken as given (no on-curve check, like pg_msm).
+ * It uses no composer state, so a sharded ctx may call it.  PG_ERR_ARG: a null pointer, log_n > 32, n_powers < 2^log_n.
+ * It synchronises the ctx stream. */
+int pg_srs_lagrange_from_powers(pg_ctx *ctx, uint32_t log_n, const pg_g1_affine *powers_of_g, uint64_t n_powers, int powers_on_device,
+                                pg_g1_affine *out, int out_on_device);
 int pg_commit_wire_evaluations(pg_ctx *ctx, uint32_t log_n, const pg_g1_affine *lagrange, uint64_t n_points, int points_on_device,
                                pg_g1_affine *out4);
 /* self-test helper: op 0: out[i] = a[i] + b[i]; op 1: out[i].x[0] = 1 if a[i] is on the curve (or infinity) else 0.  Host buffers. */

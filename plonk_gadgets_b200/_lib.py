@@ -46,7 +46,7 @@ class pg_check_stats(C.Structure):
     _fields_ = [("launches", C.c_uint64 * 8), ("rows", C.c_uint64 * 8)]
 
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 # every symbol include/pg_b200.h declares: name -> (restype, argtypes)
 _vp, _u64, _i32, _u32 = C.c_void_p, C.c_uint64, C.c_int, C.c_uint32
@@ -104,6 +104,7 @@ SIGNATURES = {
     "pg_g1_fixed_base_mul": (_i32, [_vp, _u64, _vp, _vp, _vp, _i32]),
     "pg_commit_wire_polynomials": (_i32, [_vp, _u32, _vp, _u64, _i32, _vp]),
     "pg_srs_lagrange": (_i32, [_vp, _vp, _vp, _u32, _vp, _i32]),
+    "pg_srs_lagrange_from_powers": (_i32, [_vp, _u32, _vp, _u64, _i32, _vp, _i32]),
     "pg_commit_wire_evaluations": (_i32, [_vp, _u32, _vp, _u64, _i32, _vp]),
     "pg_g1_op": (_i32, [_vp, _i32, _u64, _vp, _vp, _vp]),
     "pg_fr_to_bytes": (_i32, [_vp, _u64, _vp, _vp, _i32]),

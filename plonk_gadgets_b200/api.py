@@ -579,6 +579,18 @@ class StandardComposer:
         self._ok(self._L.pg_srs_lagrange(self._ctx, b.ctypes.data_as(C.c_void_p), bptr, log_n, res.ctypes.data_as(C.c_void_p), 0), "pg_srs_lagrange")
         return res
 
+    def srs_lagrange_from_powers(self, powers, log_n: int, out=None):
+        """Lagrange-basis SRS of the domain 2^log_n from the monomial powers alone: out[i] = (1/n) sum_j w^(-ij) powers[j] over the
+        first n = 2^log_n powers (a group inverse FFT; equals srs_lagrange(beta, log_n) when powers[j] = beta^j * G).  powers: (m, 12)
+        uint64 on the host or a device tensor; out: a device tensor to fill, else a new (n, 12) host array is returned."""
+        pp, pdev, m, _keep = self._points(powers)
+        if out is not None:
+            self._ok(self._L.pg_srs_lagrange_from_powers(self._ctx, log_n, pp, m, pdev, C.c_void_p(out.data_ptr()), 1), "pg_srs_lagrange_from_powers")
+            return out
+        res = np.zeros((1 << log_n, 12), dtype=np.uint64)
+        self._ok(self._L.pg_srs_lagrange_from_powers(self._ctx, log_n, pp, m, pdev, res.ctypes.data_as(C.c_void_p), 0), "pg_srs_lagrange_from_powers")
+        return res
+
     def commit_wire_evaluations(self, lagrange, log_n: int | None = None) -> np.ndarray:
         """(4, 12) uint64: the commitments of commit_wire_polynomials, computed from the wire values against a Lagrange-basis SRS."""
         log_n = self.domain_log_size() if log_n is None else log_n

@@ -37,6 +37,7 @@
 #include "ntt.cuh"
 #include "scan.cuh"
 #include "msm.cuh"
+#include "g1fft.cuh"
 
 namespace pg {
 
@@ -2026,7 +2027,7 @@ public:
         return rc;
     }
     // out[i] = L_i(beta) * base, i < 2^log_n: the Lagrange-basis form of the SRS for that domain (test / local setups that know
-    // beta, like PublicParameters::setup; deriving it from monomial powers alone needs a group FFT, not built)
+    // beta, like PublicParameters::setup; srs_lagrange_from_powers derives the same points from the monomial powers alone)
     int srs_lagrange(const pg_fr* beta, const pg_g1_affine* base, uint32_t log_n, pg_g1_affine* out, int out_on_device) {
         if (!beta || !out || log_n > NTT_TWO_ADICITY) return fail(PG_ERR_ARG, "srs_lagrange: null argument or domain larger than 2^32");
         const uint64_t n = 1ull << log_n;
@@ -2044,6 +2045,42 @@ public:
         a.c = fr_mul(z, fr_inv_fermat(fr_to_mont(raw)));
         if (!be.template run_simple<LagrangeScalarsBody>(a, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "lagrange scalar kernel");
         if ((rc = g1_fixed_base_mul_dev(n, base, sc, out, out_on_device))) return rc;
+        if (!be.sync()) return fail(PG_ERR_CUDA, "sync");
+        release_scratch_from(mark);
+        return PG_OK;
+    }
+    // out[i] = (1/n) sum_j w^(-ij) powers[j], i < n = 2^log_n: the Lagrange-basis SRS from the first n monomial powers, by the group
+    // inverse FFT of g1fft.cuh.  For powers[j] = beta^j * base it is srs_lagrange(beta, base, log_n), point for point.
+    int srs_lagrange_from_powers(uint32_t log_n, const pg_g1_affine* powers, uint64_t n_powers, int powers_on_device, pg_g1_affine* out, int out_on_device) {
+        if (!powers || !out || log_n > NTT_TWO_ADICITY) return fail(PG_ERR_ARG, "srs_lagrange_from_powers: null argument or domain larger than 2^32");
+        const uint64_t n = 1ull << log_n;
+        if (n_powers < n) return fail(PG_ERR_ARG, "srs_lagrange_from_powers: the SRS holds fewer powers than the domain size");
+        const size_t mark = scratch.size();
+        auto tmp = [&](size_t bytes) -> uint4* { void* q = dalloc(bytes); if (q) scratch.push_back(q); return (uint4*)q; };
+        int rc; const uint4* dp = stage_bytes(powers, n * sizeof(pg_g1_affine), powers_on_device, &rc); if (!dp) return rc;
+        if (log_n == 0) rc = deliver(out, dp, sizeof(pg_g1_affine), out_on_device);          // L_0 = 1
+        else {
+            if ((rc = ntt_twiddles(log_n))) return rc;
+            uint4* data = tmp(n * sizeof(G1X));
+            uint4* d_out = out_on_device ? reinterpret_cast<uint4*>(out) : tmp(n * sizeof(pg_g1_affine));
+            const uint64_t tile = std::min<uint64_t>(n, FB_TILE);
+            uint4* prefix = tmp(tile * sizeof(Fp));
+            if (!data || !d_out || !prefix) return fail(PG_ERR_OOM, "group FFT buffers");
+            Fr raw = fr_zero(); raw.v[0] = (uint32_t)n; raw.v[1] = (uint32_t)(n >> 32);
+            G1FftIngestBody::Args ia{dp, data, n, log_n, fr_from_mont(fr_inv_fermat(fr_to_mont(raw)))};
+            if (!be.template run_simple<G1FftIngestBody>(ia, n, CLS_OTHER)) return fail(PG_ERR_CUDA, "group FFT ingest kernel");
+            for (uint32_t s = 0; s < log_n; s++) {
+                G1FftStageBody::Args sa{data, ntt_tw, n >> 1, log_n, s};
+                if (!be.template run_simple<G1FftStageBody>(sa, sa.n, CLS_OTHER)) return fail(PG_ERR_CUDA, "group FFT stage kernel");
+            }
+            for (uint64_t i0 = 0; i0 < n; i0 += tile) {
+                const uint64_t cnt = std::min<uint64_t>(tile, n - i0), threads = (cnt + FB_CHUNK - 1) / FB_CHUNK;
+                G1BatchAffineBody::Args na{data + 12 * i0, prefix, d_out + 6 * i0, threads, cnt};
+                if (!be.template run_simple<G1BatchAffineBody>(na, threads, CLS_OTHER)) return fail(PG_ERR_CUDA, "group FFT normalisation kernel");
+            }
+            if (!out_on_device) rc = deliver(out, d_out, n * sizeof(pg_g1_affine), 0);
+        }
+        if (rc) return rc;
         if (!be.sync()) return fail(PG_ERR_CUDA, "sync");
         release_scratch_from(mark);
         return PG_OK;

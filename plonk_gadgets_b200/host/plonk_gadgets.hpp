@@ -221,6 +221,12 @@ public:
         ok(pg_srs_lagrange(ctx_, reinterpret_cast<const pg_fr*>(&beta), nullptr, log_n, out.data(), 0), "pg_srs_lagrange");
         return out;
     }
+    /// the same form from the monomial powers alone (a trusted setup's powers_of_g, beta unknown): the first 2^log_n powers are read
+    std::vector<pg_g1_affine> srs_lagrange_from_powers(const std::vector<pg_g1_affine>& powers_of_g, uint32_t log_n) {
+        std::vector<pg_g1_affine> out((size_t)1 << log_n);
+        ok(pg_srs_lagrange_from_powers(ctx_, log_n, powers_of_g.data(), powers_of_g.size(), 0, out.data(), 0), "pg_srs_lagrange_from_powers");
+        return out;
+    }
     /// the same four commitments as commit_wire_polynomials, from the wire values against the Lagrange-basis SRS (no FFT)
     std::vector<pg_g1_affine> commit_wire_evaluations(const std::vector<pg_g1_affine>& lagrange, uint32_t log_n) {
         std::vector<pg_g1_affine> out(4);
