@@ -372,6 +372,7 @@ struct CheckArgs {
     DevTab tab[MAX_TABS];
     const uint4* param; uint64_t param_stride;
     const DevRow* rows; const uint32_t* pool;
+    const Fr* fold;                  // fr_fold_constants of every q_m of the template, 8 per entry (DevRow::fold)
     uint32_t n_rows, n_pool;
     uint64_t n_inst; uint64_t base_row;
     unsigned long long* counters;
@@ -383,10 +384,10 @@ struct SparseProg { const SpOp* ops; uint32_t n; };
 struct CheckProgArgs { CheckArgs a; SparseProg prog; };      // one argument block for k_check_prog
 
 // GENERIC mode evaluates  a*(q_m*b + q_l) + q_r*b + q_o*c + q_4*d + q_c + PI  -- the gate polynomial with the bilinear term
-// factored, five multiplications instead of six, still without looking at any selector value: one Montgomery
-// multiplication u = q_m*b (fully reduced, + q_l without reduction), then the four remaining products as ONE dot product with
-// a single interleaved reduction (fr_dot_wide): 64+48 + 4*64+48 = 416 wide multiplier instructions per row instead of
-// 6*(64+64).  The 9-limb result plus q_c and PI is tested for "0 mod q" directly.
+// factored, five multiplications instead of six, still without looking at any selector value: u = q_m*b through the eight
+// constants the host folded from q_m (fr_mul_folded: 64 products and two reduction steps, u < q + 2^227, + q_l without reduction),
+// then the four remaining products as ONE dot product with a single interleaved reduction (fr_dot_wide): 64+12 + 4*64+48 = 380
+// wide multiplier instructions per row instead of 6*(64+64).  The 9-limb result plus q_c and PI is tested for "0 mod q" directly.
 // SPARSE mode: structure-aware, see sparse_terms.
 struct CheckBody {
     typedef CheckArgs Args;
@@ -446,8 +447,10 @@ struct CheckBody {
         }
     }
 
-    // gate equation of row `row` for instance i: true iff it holds
-    template <int MODE, class PoolT>
+    // gate equation of row `row` for instance i: true iff it holds.  FOLD: q_m*b through fr_mul_folded (kernels with a budget of at
+    // least 96 registers); otherwise through fr_mul_eo -- the fold constants in flight make the kernels of 64..85 registers and the
+    // range-widget kernels spill more than they do
+    template <int MODE, bool FOLD = true, class PoolT>
     PG_HD static bool row_holds(const Args& a, const DevRow& row, const PoolT& pool, const QRegs& q, uint64_t i) {
         if (MODE != 0) return row_holds_sparse(a, row, pool, q, i);
         Fr w[5];
@@ -455,7 +458,8 @@ struct CheckBody {
         for (int k = 0; k < 4; k++) w[k + 1] = row_load(row, k, i);
         uint32_t t[9];
         Fr sel[4];
-        sel[0] = fr_add_noreduce(fr_mul_eo(pool(row.sel[0]), w[2], q), pool(row.sel[1]));   // q_m*b + q_l  (< 2q < 2^256)
+        const Fr qmb = FOLD ? fr_mul_folded(a.fold + 8 * (uint32_t)row.fold, w[2], q) : fr_mul_eo(pool(row.sel[0]), w[2], q);
+        sel[0] = fr_add_noreduce(qmb, pool(row.sel[1]));                                     // q_m*b + q_l  (< 2q + 2^227 < 2^256)
 #pragma unroll
         for (int k = 1; k < 4; k++) sel[k] = pool(row.sel[k + 1]);                           // q_r q_o q_4
         fr_dot_wide<4>(t, w + 1, sel, q);                                                     // a*u + b*q_r + c*q_o + d*q_4
@@ -491,7 +495,7 @@ struct CheckBody {
         return limbs9_is_multiple_of_q(t);
     }
     // evaluates all rows of instance i; returns the number of unsatisfied rows, updates first_bad (global row index)
-    template <int MODE, class PoolT>
+    template <int MODE, bool FOLD = true, class PoolT>
     PG_HD static uint32_t run(const Args& a, const PoolT& pool, const QRegs& q, uint64_t i, unsigned long long& first_bad) {
         uint32_t bad = 0;
         // (No prefetch of the next row's wires: requesting them into L1 one row ahead -- eight more warp-uniform loads of the next
@@ -499,7 +503,7 @@ struct CheckBody {
         // costs 2.7 % on the leaner row loop of run r05e: 256.2 -> 249.3 ms, run r05n.  Twenty resident warps per SM hide the loads.)
         for (uint32_t r = 0; r < a.n_rows; r++) {
             const DevRow row = a.rows[r];
-            if (!row_holds<MODE>(a, row, pool, q, i)) {
+            if (!row_holds<MODE, FOLD>(a, row, pool, q, i)) {
                 bad++;
                 const unsigned long long g = a.base_row + i * (uint64_t)a.n_rows + r;
                 if (g < first_bad) first_bad = g;
@@ -714,7 +718,7 @@ struct CheckRowsBody {
 
 // Segments that hold rows of another widget (GATE_RANGE / GATE_NONE, layout.h): one thread per (row, instance), lanes = instances
 // (kernels.cuh k_check_gates).
-//   arithmetic rows: the generic kernel's row evaluation (CheckBody::row_holds<0>);
+//   arithmetic rows: the generic kernel's row evaluation (CheckBody::row_holds<0>, with q_m*b through fr_mul_eo);
 //   range rows     : q_range*(D(c - 4d) + D(b - 4c) + D(a - 4b) + D(d_next - 4a)), D(f) = f(f-1)(f-2)(f-3), with d_next the fourth
 //                    wire of the NEXT row [dusk-plonk check_circuit_satisfied / range widget, recalled].  Evaluated as
 //                    D(f) = u^2 - 1, u = f(f-3) + 1  (f(f-3) = g, (f-1)(f-2) = g + 2, g(g+2) = (g+1)^2 - 1): four multiplications,
@@ -763,7 +767,7 @@ struct GateRowsCheckBody {
     }
     template <class PoolT>
     PG_HD static bool arith_row_holds(const CheckArgs& a, const DevRow& row, const PoolT& pool, const QRegs& q, uint64_t i) {
-        return a.mode != 0 ? CheckBody::row_holds_sparse(a, row, pool, q, i) : CheckBody::row_holds<0>(a, row, pool, q, i);
+        return a.mode != 0 ? CheckBody::row_holds_sparse(a, row, pool, q, i) : CheckBody::row_holds<0, false>(a, row, pool, q, i);
     }
     template <class PoolT>
     PG_HD static bool row_ok(const CheckArgs& a, const PoolT& pool, const QRegs& q, uint32_t r, uint64_t i) {

@@ -50,7 +50,7 @@ struct Segment {
     Template t;
     uint64_t n_inst = 0, n_alloc = 0, base_row = 0, base_var = 0;
     uint4* fr = nullptr; uint32_t* bits = nullptr; uint4* param = nullptr;
-    DevRow* d_rows = nullptr; uint32_t* d_varloc = nullptr; uint32_t* d_pool = nullptr;   // views into d_image
+    DevRow* d_rows = nullptr; uint32_t* d_varloc = nullptr; uint32_t* d_pool = nullptr; Fr* d_fold = nullptr;   // views into d_image
     void* d_image = nullptr;
     DevTab tabs[MAX_TABS] = {};
     std::vector<DevRow> rows;
@@ -351,7 +351,8 @@ public:
     // Appends a segment of n instances of template t whose operands are the given columns.  Allocates the variable
     // table, resolves the symbolic wires and uploads the row program.  The witness kernels run afterwards.
     static size_t image_bytes_bound(const Template& T) {      // upper bound of a segment image (the structure-aware program has at most ~12 operations per row)
-        return (T.rows.size() * (sizeof(DevRow) + 12 * sizeof(SpOp)) + T.var_loc.size() * sizeof(uint32_t) + (T.pool.size() + 8 * T.rows.size()) * sizeof(Fr) + 255) & ~(size_t)255;
+        const size_t fold = 8 * std::min(T.rows.size(), T.pool.size());     // fold table: 8 constants per distinct q_m
+        return (T.rows.size() * (sizeof(DevRow) + 12 * sizeof(SpOp)) + T.var_loc.size() * sizeof(uint32_t) + (T.pool.size() + 8 * T.rows.size() + fold) * sizeof(Fr) + 255) & ~(size_t)255;
     }
     int push_segment(Template&& t, uint64_t n, const Column* operands, uint32_t n_operands, const SegmentView* view = nullptr, CachedRange* cache = nullptr) {
         Segment s;
@@ -376,6 +377,8 @@ public:
             s.rows = cache->rows; s.sp_ops = cache->sp_ops; s.t.pool = cache->pool; img = cache->img;
         } else {
         s.rows.resize(T.rows.size());
+        std::map<uint16_t, uint16_t> fold_of;        // q_m pool index -> its entry in the fold table (order of first use)
+        std::vector<Fr> fold;
         for (size_t r = 0; r < T.rows.size(); r++) {
             const RowT& src = T.rows[r]; DevRow d; memset(&d, 0, sizeof(d));
             for (int w = 0; w < 4; w++) {
@@ -386,6 +389,13 @@ public:
             }
             for (int k = 0; k < 6; k++) d.sel[k] = src.sel[k];
             d.pi_sel = src.pi_sel; d.qc_param = src.qc_param; d.pi_param = src.pi_param; d.gate = src.gate;
+            auto f = fold_of.find(src.sel[0]);
+            if (f == fold_of.end()) {
+                f = fold_of.emplace(src.sel[0], (uint16_t)fold_of.size()).first;
+                fold.resize(fold.size() + 8);
+                fr_fold_constants(&fold[fold.size() - 8], T.pool[src.sel[0]]);
+            }
+            d.fold = f->second;
             if (src.gate != GATE_ARITH) s.other_gates = true;
             for (int w = 0; w < 4; w++) {            // instance-0 address of each wire value (see DevRow::addr)
                 const uint32_t kind = loc_kind(d.loc[w]), pay = loc_payload(d.loc[w]);
@@ -397,11 +407,13 @@ public:
             s.rows[r] = d;
         }
         if (cfg.check_mode == PG_CHECK_SPARSE && !s.other_gates) build_sparse_program(s);   // segments with range rows have their own check body
-        // rows | variable map | selector pool | structure-aware program go up in ONE copy (one staging image per segment)
+        // rows | variable map | selector pool | fold table | structure-aware program go up in ONE copy (one staging image per segment);
+        // every section starts 32-byte aligned (fr_load_fold reads the fold table with 256-bit loads)
         const size_t b_rows0 = s.rows.size() * sizeof(DevRow), b_var0 = (T.var_loc.size() * sizeof(uint32_t) + 31) & ~(size_t)31, b_pool0 = T.pool.size() * sizeof(Fr);
-        const size_t b_sp0 = s.sp_ops.size() * sizeof(SpOp);
-        img.resize(b_rows0 + b_var0 + b_pool0 + b_sp0);
-        if (b_sp0) memcpy(img.data() + b_rows0 + b_var0 + b_pool0, s.sp_ops.data(), b_sp0);
+        const size_t b_fold0 = fold.size() * sizeof(Fr), b_sp0 = s.sp_ops.size() * sizeof(SpOp);
+        img.resize(b_rows0 + b_var0 + b_pool0 + b_fold0 + b_sp0);
+        if (b_sp0) memcpy(img.data() + b_rows0 + b_var0 + b_pool0 + b_fold0, s.sp_ops.data(), b_sp0);
+        if (b_fold0) memcpy(img.data() + b_rows0 + b_var0 + b_pool0, fold.data(), b_fold0);
         if (b_rows0) memcpy(img.data(), s.rows.data(), b_rows0);
         if (!T.var_loc.empty()) memcpy(img.data() + b_rows0, T.var_loc.data(), T.var_loc.size() * sizeof(uint32_t));
         memcpy(img.data() + b_rows0 + b_var0, T.pool.data(), b_pool0);
@@ -417,7 +429,8 @@ public:
         s.d_rows = b_rows ? (DevRow*)d_img : nullptr;
         s.d_varloc = T.var_loc.empty() ? nullptr : (uint32_t*)(d_img + b_rows);
         s.d_pool = (uint32_t*)(d_img + b_rows + b_var);
-        s.d_sp = b_sp ? (SpOp*)(d_img + b_rows + b_var + b_pool) : nullptr;
+        s.d_fold = (Fr*)(d_img + b_rows + b_var + b_pool);       // the fold table fills the image up to the program
+        s.d_sp = b_sp ? (SpOp*)(d_img + img.size() - b_sp) : nullptr;
         s.d_image = d_img;
         // (pageable sources: cudaMemcpyAsync has consumed them when it returns; they stay alive in the Segment anyway)
         segs.push_back(std::move(s));
@@ -808,7 +821,7 @@ public:
             if (s.fused_ok && skip_fused) continue;  // verdict already in CNT_FUSED_* (pg_check adds it; a sharded check renumbers rows and evaluates them again)
             CheckArgs a; memset(&a, 0, sizeof(a));
             for (int j = 0; j < MAX_TABS; j++) a.tab[j] = s.tabs[j];
-            a.param = s.param; a.param_stride = s.n_alloc; a.rows = s.d_rows; a.pool = s.d_pool;
+            a.param = s.param; a.param_stride = s.n_alloc; a.rows = s.d_rows; a.pool = s.d_pool; a.fold = s.d_fold;
             a.n_rows = (uint32_t)s.t.rows.size(); a.n_pool = (uint32_t)s.t.pool.size();
             a.n_inst = s.n_inst; a.base_row = (mine && k > 0) ? mine[k - 1].row_base : s.base_row; a.counters = d_counters; a.mode = cfg.check_mode;
             if (s.other_gates) {                     // rows of the range widget: per-row body, one thread per (row, instance)

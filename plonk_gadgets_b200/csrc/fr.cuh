@@ -296,6 +296,7 @@ inline void mad_row_shift(uint32_t* o, uint32_t& e0, uint32_t x0, uint32_t x2, u
 inline void merge_even_odd(uint32_t* r, const uint32_t* e, const uint32_t* o) {
     uint64_t c = 0;
     for (int i = 0; i < 7; i++) { uint64_t s = (uint64_t)e[i] + o[i + 1] + c; r[i] = (uint32_t)s; c = s >> 32; }
+    if ((uint64_t)e[7] + c > 0xffffffffull) PG_EMU_VIOLATION();   // the result must fit 256 bits
     r[7] = e[7] + (uint32_t)c;
 }
 #endif
@@ -499,7 +500,9 @@ PG_HD void dot_step(uint32_t* X, uint32_t* Y, uint32_t& z, const Fr* a, const ui
     }
     dred_rows(X, Y, z, q);
 }
-// r[0..8] = (sum_p a[p]*b[p]) / 2^256 mod q up to a multiple of q, r < (K+1)*q + 2^224.  a[p], b[p] < 2q.
+// r[0..8] = (sum_p a[p]*b[p]) / 2^256 mod q up to a multiple of q:  r = (sum_p a[p]*b[p] + M*q) / 2^256 with M < 2^256, so
+// r < q + sum_p a[p]*b[p] / 2^256  -- r < (K+1)*q for a[p] < q and any 256-bit b[p] (the generic row's u = q_m*b + q_l < 2q + 2^227),
+// r < (2K+1)*q for a[p] < 2q, b[p] < 2q.
 template <int K>
 PG_HD void fr_dot_wide(uint32_t* r, const Fr* a, const Fr* b, const QRegs& q) {
     uint32_t even[8], odd[8], z, bi[K];
@@ -519,6 +522,68 @@ PG_HD void fr_dot_wide(uint32_t* r, const Fr* a, const Fr* b, const QRegs& q) {
 }
 template <int K>
 PG_HD void fr_dot_wide(uint32_t* r, const Fr* a, const Fr* b) { fr_dot_wide<K>(r, a, b, q_regs_default()); }
+
+// ---- q_m*b with the reduction folded into per-selector constants -------------------------------------------------------
+// For a selector s = q_m*R (Montgomery form) the host precomputes C[i] = q_m * 2^(32i+64) mod q, i = 0..7 (fr_fold_constants).
+// For b as stored (any 256-bit value, limbs b[i])  U = sum_i b[i]*C[i]  is congruent to q_m*b*2^64: eight product rows at the same
+// offset with no reduction between them (U < 8*2^32*q < 2^290: the ten limbs X | Y | z of the dot product).  Two Montgomery steps
+// (m = -T[0], T += m*q, T >>= 32) leave  r == q_m*b == fr_mul_eo(s, b) (mod q)  with  r < q + 2^227:  8*8 + 2*6 = 76 wide products
+// instead of fr_mul_eo's 112, and no conditional subtraction.  The result is NOT reduced.
+#if defined(__CUDA_ARCH__)
+// division by 2^32 between two reduction steps (o[0] == 0):  e0 += o[1];  o <- (o >> 2 limbs | z at the top), the odd array of the next step
+PG_D void dshift_rows(uint32_t* o, uint32_t& e0, uint32_t z) {
+    asm("add.cc.u32 %8, %8, %1;\n\taddc.cc.u32 %0, %2, 0;\n\taddc.cc.u32 %1, %3, 0;\n\taddc.cc.u32 %2, %4, 0;\n\taddc.cc.u32 %3, %5, 0;\n\t"
+        "addc.cc.u32 %4, %6, 0;\n\taddc.cc.u32 %5, %7, 0;\n\taddc.u32 %6, 0, 0;"
+        : "+r"(o[0]), "+r"(o[1]), "+r"(o[2]), "+r"(o[3]), "+r"(o[4]), "+r"(o[5]), "+r"(o[6]), "+r"(o[7]), "+r"(e0));
+    o[7] = z;
+}
+// one 256-bit load of a fold constant (the table is 32-byte aligned and read-only while a kernel runs)
+PG_D Fr fr_load_fold(const Fr* p) {
+    Fr r;
+    asm("ld.global.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+        : "=r"(r.v[0]), "=r"(r.v[1]), "=r"(r.v[2]), "=r"(r.v[3]), "=r"(r.v[4]), "=r"(r.v[5]), "=r"(r.v[6]), "=r"(r.v[7]) : "l"(p));
+    return r;
+}
+#else
+inline void dshift_rows(uint32_t* o, uint32_t& e0, uint32_t z) {
+    if (o[0] != 0) PG_EMU_VIOLATION();                                  // the reduction must have cleared the lowest limb
+    const uint64_t s = (uint64_t)e0 + o[1]; e0 = (uint32_t)s;
+    uint64_t c = s >> 32;
+    for (int k = 0; k < 6; k++) { const uint64_t t = (uint64_t)o[k + 2] + c; o[k] = (uint32_t)t; c = t >> 32; }
+    o[6] = (uint32_t)c; o[7] = z;
+}
+inline Fr fr_load_fold(const Fr* p) { return *p; }
+#endif
+// C[0..7] for the selector s (Montgomery form, < q): C[i] = mont(s, 2^(32i+64) mod q) = q_m * 2^(32i+64) mod q
+PG_HD void fr_fold_constants(Fr* C, const Fr& s) {
+    Fr p = {{0, 0, 1, 0, 0, 0, 0, 0}};                                     // 2^64 (a plain value below q)
+    const Fr two32 = {{0, 1, 0, 0, 0, 0, 0, 0}};
+    const Fr step = fr_mul_cios(two32, fr_r2());                           // 2^32*R: a Montgomery product with it multiplies by 2^32
+    for (int i = 0; i < 8; i++) { C[i] = fr_mul_cios(s, p); p = fr_mul_cios(p, step); }
+}
+// r == s*b*R^-1 (mod q), r < q + 2^227, for the constants C = fr_fold_constants(s) (device: global memory) and any 256-bit b
+PG_HD Fr fr_mul_folded(const Fr* C, const Fr& b, const QRegs& q) {
+    uint32_t X[8], Y[8], z = 0;
+    // One constant ahead: the address of C[p+1] is ORed with z >> 3, which is 0 (z < 8 after every row: U < 2^290) but not to ptxas, so
+    // the load cannot be hoisted above row p-1.  Without it ptxas issues all eight loads early and k_check<0,0> spills at 96 registers.
+    // (An OR on the low address word is one logic instruction; an added index would become an IMAD.WIDE on the multiplier pipe.)
+    Fr c = fr_load_fold(C), cn = fr_load_fold(C + 1);
+    mul_row(Y, c.v[1], c.v[3], c.v[5], c.v[7], b.v[0]);
+    mul_row(X, c.v[0], c.v[2], c.v[4], c.v[6], b.v[0]);
+#pragma unroll
+    for (int p = 1; p < 8; p++) {
+        c = cn;
+        if (p < 7) cn = fr_load_fold(reinterpret_cast<const Fr*>(reinterpret_cast<uintptr_t>(C + p + 1) | (z >> 3)));
+        dmad_row_y(Y, z, c.v[1], c.v[3], c.v[5], c.v[7], b.v[p]);
+        dmad_row_x(X, Y[7], z, c.v[0], c.v[2], c.v[4], c.v[6], b.v[p]);
+    }
+    dred_rows(X, Y, z, q);             // T = U + m*q < 2^291
+    dshift_rows(X, Y[0], z);           // T >>= 32 (< 2^259): Y even, X odd
+    red_rows(Y, X, q);                 // T + m*q < 2^288: nothing leaves limb 8
+    Fr r;
+    merge_even_odd(r.v, X, Y);         // (X + Y>>32), Y[0] == 0
+    return r;
+}
 // plain 256-bit addition a + b (no reduction); the caller guarantees a + b < 2^256 (e.g. both < q)
 PG_HD Fr fr_add_noreduce(const Fr& a, const Fr& b) {
     Fr r;

@@ -180,7 +180,7 @@ __global__ void __launch_bounds__(CheckShape<SHAPE>::BLOCK_T, CheckShape<SHAPE>:
     uint32_t bad = 0;
     if (i < a.n_inst) {
         SmemPool pool = {s_pool, s_kq};
-        bad = CheckBody::run<MODE>(a, pool, q, i, first_bad);
+        bad = CheckBody::run<MODE, 65536 / (CHECK_BLOCK * CheckShape<SHAPE>::MIN_BLOCKS) >= 96>(a, pool, q, i, first_bad);   // FOLD: >= 96 registers
     }
     // warp-level reduction, then one atomic per warp that saw a violation
 #pragma unroll

@@ -50,7 +50,8 @@ struct DevRow {               // 96 bytes
     int16_t qc_param;         // >= 0: q_c is param slot qc_param of the instance (sel[5] ignored)
     int16_t pi_param;         // >= 0: PI is param slot pi_param of the instance
     uint16_t gate;            // GATE_ARITH (q_arith = 1), GATE_RANGE (q_range = 1, q_arith = 0) or GATE_NONE (both 0)
-    uint16_t pad[6];
+    uint16_t fold;            // entry of the segment's fold table that belongs to q_m (fr_mul_folded's eight constants)
+    uint16_t pad[5];
     // pre-resolved device address of instance 0 of each wire value (FR: the 32-byte scalar; BIT: the 32-bit word holding the
     // bit; ZERO: 0).  The gate-check kernel adds i*32 (or i*4) and never touches the table descriptors: no per-row
     // slot*stride products on the multiplier pipe.
