@@ -373,6 +373,7 @@ struct CheckArgs {
     const uint4* param; uint64_t param_stride;
     const DevRow* rows; const uint32_t* pool;
     const Fr* fold;                  // fr_fold_constants of every q_m of the template, 8 per entry (DevRow::fold)
+    const uint4* bfold;              // byte_fold_block of every q_r / q_o / q_4 of the template, BF_BYTES each (DevRow::bfold; generic mode)
     uint32_t n_rows, n_pool;
     uint64_t n_inst; uint64_t base_row;
     unsigned long long* counters;
@@ -388,6 +389,8 @@ struct CheckProgArgs { CheckArgs a; SparseProg prog; };      // one argument blo
 // constants the host folded from q_m (fr_mul_folded: 64 products and two reduction steps, u < q + 2^227, + q_l without reduction),
 // then the four remaining products as ONE dot product with a single interleaved reduction (fr_dot_wide): 64+12 + 4*64+48 = 380
 // wide multiplier instructions per row instead of 6*(64+64).  The 9-limb result plus q_c and PI is tested for "0 mod q" directly.
+// This is the reference the tests compare against and the body of the small-segment, tuning-shape and range-widget kernels; large
+// generic segments run k_check_tc (kernels.cuh), which takes q_r*b + q_o*c + q_4*d to the tensor cores.
 // SPARSE mode: structure-aware, see sparse_terms.
 struct CheckBody {
     typedef CheckArgs Args;

@@ -75,7 +75,8 @@ public:
     }
     template <int SHAPE>
     bool set_check_attrs() {
-        PG_CUDA(cudaFuncSetAttribute(k_check<0, SHAPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+        if constexpr (SHAPE == 0) PG_CUDA(cudaFuncSetAttribute(k_check_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+        else PG_CUDA(cudaFuncSetAttribute(k_check<0, SHAPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         PG_CUDA(cudaFuncSetAttribute(k_check<1, SHAPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         PG_CUDA(cudaFuncSetAttribute(k_check_prog<SHAPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         return true;
@@ -86,6 +87,7 @@ public:
         const unsigned grid = (unsigned)((a.n_inst + T - 1) / T);
         if (a.mode == PG_CHECK_SPARSE && prog.ops) { const CheckProgArgs pa{a, prog}; k_check_prog<SHAPE><<<grid, T, smem, stream>>>(pa); }   // compiled row program
         else if (a.mode == PG_CHECK_SPARSE) k_check<1, SHAPE><<<grid, T, smem, stream>>>(a);
+        else if constexpr (SHAPE == 0) k_check_tc<<<grid, T, smem, stream>>>(a);   // generic mode, default shape: tensor-core selector products
         else k_check<0, SHAPE><<<grid, T, smem, stream>>>(a);
     }
     void shutdown() {

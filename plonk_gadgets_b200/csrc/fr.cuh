@@ -584,6 +584,51 @@ PG_HD Fr fr_mul_folded(const Fr* C, const Fr& b, const QRegs& q) {
     merge_even_odd(r.v, X, Y);         // (X + Y>>32), Y[0] == 0
     return r;
 }
+// ---- the tensor-core part of the generic row: columns of the byte product -------------------------------------------------
+// k_check_tc computes q_r*b + q_o*c + q_4*d (times R^-1, up to a multiple of q) as 32 s32 columns c[j] = sum over the 96 wire bytes
+// of byte * (byte j of a byte-fold constant), c[j] <= 96*255*255 < 2^23, standing for L = sum_j c[j]*2^(8j) < 96*255*q.
+// t[0..8] += L without a product:  P_k = c[4k] + (c[4k+1] << 8) and D_k = c[4k+2] + (c[4k+3] << 8) fit 32 bits, and
+// L = sum_k P_k*2^(32k) + sum_k D_k*2^(32k+16), whose second sum has the limbs G_k = (D_k << 16) | (D_(k-1) >> 16):
+// two 9-limb additions.
+PG_HD void add_byte_columns(uint32_t* t, const uint32_t* c) {
+    Fr P, G;
+    uint32_t dprev = 0;
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+#if !defined(__CUDA_ARCH__)
+        for (int j = 0; j < 4; j++) if (c[4 * k + j] >= (1u << 23)) PG_EMU_VIOLATION();   // the column bound the split relies on
+#endif
+#if defined(__CUDA_ARCH__)
+        // x + (y << 8) written as a funnel shift: one LEA.HI on the integer ALU (as a shift and an add ptxas makes it an IMAD, which
+        // would take the multiplier pipe the rest of the row is bound by)
+        P.v[k] = c[4 * k] + __funnelshift_l(0u, c[4 * k + 1], 8);
+        const uint32_t d = c[4 * k + 2] + __funnelshift_l(0u, c[4 * k + 3], 8);
+        G.v[k] = __funnelshift_l(dprev, d, 16);
+#else
+        P.v[k] = c[4 * k] + (c[4 * k + 1] << 8);
+        const uint32_t d = c[4 * k + 2] + (c[4 * k + 3] << 8);
+        G.v[k] = (d << 16) | (dprev >> 16);
+#endif
+        dprev = d;
+    }
+    add9_fr(t, P);
+    add9_fr(t, G);
+#if !defined(__CUDA_ARCH__)
+    if (t[8] + (dprev >> 16) < t[8]) PG_EMU_VIOLATION();
+#endif
+    t[8] += dprev >> 16;                                          // G_8
+}
+// t == 0 (mod q) for a 9-limb t < 2^15*q: since q = 1 (mod 2^32), t is a multiple of q iff t == k*q for k = t[0] < 2^15.
+// k*q by eight wide products (k*q_i + carry is one IMAD.WIDE.U32 with a 64-bit addend each).
+PG_HD bool limbs9_is_small_multiple_of_q(const uint32_t* t, const QRegs& q) {
+    const uint32_t k = t[0] & 0x7fffu;
+    uint32_t diff = t[0] >> 15;
+    uint64_t c = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) { c = (uint64_t)q.v[i] * k + (c >> 32); diff |= (uint32_t)c ^ t[i]; }
+    diff |= (uint32_t)(c >> 32) ^ t[8];
+    return diff == 0;
+}
 // plain 256-bit addition a + b (no reduction); the caller guarantees a + b < 2^256 (e.g. both < q)
 PG_HD Fr fr_add_noreduce(const Fr& a, const Fr& b) {
     Fr r;

@@ -195,6 +195,154 @@ __global__ void __launch_bounds__(CheckShape<SHAPE>::BLOCK_T, CheckShape<SHAPE>:
     }
 }
 
+// ---- generic gate check with q_r*b + q_o*c + q_4*d on the tensor cores ----------------------------------------------------------
+// One instance per thread, 128 threads per block, the row template walked by the whole block in lock step.  For one row the three
+// selector-times-wire products of the block's 128 instances are ONE u8 contraction (layout.h, byte-fold blocks):
+//     C (128 x 32, s32) = A (128 x 96, u8: bytes of b | c | d) x B (96 x 32, u8: the blocks of q_r; q_o; q_4)
+// three tcgen05.mma.kind::i8 of M = 128, N = 32, K = 32 into 32 tensor-memory columns.  The threads write A, the row's three blocks
+// are copied into B (cp.async), one thread issues the MMAs; meanwhile every thread evaluates a*(q_m*b + q_l) on the integer pipe
+// (fr_mul_folded, fr_dot_wide<1>: 76 + 64 + 48 wide products), then reads its own accumulator lane, adds the columns
+// (add_byte_columns: no product) and q_c + PI, and tests the sum (< 24484*q) with limbs9_is_small_multiple_of_q (8 products).
+// The verdict is exact for every input, and every row does the same work whatever its selector values.
+// One A / B / accumulator buffer: a thread writes row r+1's operands only after it has seen row r's MMA complete (mbarrier), and the
+// MMA of row r+1 is issued after the block barrier that follows every thread's read of row r's accumulator.
+constexpr int TC_BLOCK = 128, TC_MIN_BLOCKS = 5;   // <= 102 registers, 20 warps/SM (the k_check<0,0> shape it replaces)
+constexpr uint32_t TC_TMEM_COLS = 32;              // one s32 accumulator of N = 32 columns
+// tcgen05.alloc waits for free columns: the blocks that can be resident on an SM (at most 2048 threads) must fit its 512 columns
+static_assert((2048 / TC_BLOCK) * TC_TMEM_COLS <= 512, "tensor-memory columns of the resident k_check_tc blocks exceed 512");
+constexpr uint32_t TC_A_LBO = TC_BLOCK * 16;       // A: 16-byte K chunk kc of instance t at kc * TC_A_LBO + t * 16 (SBO 128 as in B)
+// instruction descriptor of kind::i8: D s32 (bits 4-5 = 2), A and B unsigned (bits 7-9, 10-12 = 0), both K-major (bits 15, 16 = 0),
+// N >> 3 at bits 17-22, M >> 4 at bits 24-28
+constexpr uint32_t TC_IDESC = (2u << 4) | ((32u >> 3) << 17) | ((128u >> 4) << 24);
+// shared-memory matrix descriptor, no swizzle: start >> 4 (bits 0-13), LBO >> 4 (16-29), SBO >> 4 (32-45), version 1 (46-47)
+__device__ __forceinline__ uint64_t tc_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
+    return (uint64_t)((saddr & 0x3ffffu) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46);
+}
+__device__ __forceinline__ void tc_mma(uint32_t tmem, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+                 ::"r"(tmem), "l"(adesc), "l"(bdesc), "r"(TC_IDESC), "r"(accumulate) : "memory");
+}
+__device__ __forceinline__ void tc_fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void mbar_wait(uint32_t mbar, uint32_t parity) {
+    uint32_t done;
+    do {
+        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+                     : "=r"(done) : "r"(mbar), "r"(parity) : "memory");
+    } while (!done);
+}
+// the 32 accumulator columns of this thread's lane (warp w reads lanes 32w .. 32w + 31)
+__device__ __forceinline__ void tc_load_columns(uint32_t* c, uint32_t taddr) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(c[0]), "=r"(c[1]), "=r"(c[2]), "=r"(c[3]), "=r"(c[4]), "=r"(c[5]), "=r"(c[6]), "=r"(c[7]),
+                   "=r"(c[8]), "=r"(c[9]), "=r"(c[10]), "=r"(c[11]), "=r"(c[12]), "=r"(c[13]), "=r"(c[14]), "=r"(c[15]) : "r"(taddr) : "memory");
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(c[16]), "=r"(c[17]), "=r"(c[18]), "=r"(c[19]), "=r"(c[20]), "=r"(c[21]), "=r"(c[22]), "=r"(c[23]),
+                   "=r"(c[24]), "=r"(c[25]), "=r"(c[26]), "=r"(c[27]), "=r"(c[28]), "=r"(c[29]), "=r"(c[30]), "=r"(c[31]) : "r"(taddr + 16) : "memory");
+    // the registers are valid only after wait::ld: tie them to it so that no use is scheduled above it
+    asm volatile("tcgen05.wait::ld.sync.aligned;"
+                 : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3]), "+r"(c[4]), "+r"(c[5]), "+r"(c[6]), "+r"(c[7]),
+                   "+r"(c[8]), "+r"(c[9]), "+r"(c[10]), "+r"(c[11]), "+r"(c[12]), "+r"(c[13]), "+r"(c[14]), "+r"(c[15]),
+                   "+r"(c[16]), "+r"(c[17]), "+r"(c[18]), "+r"(c[19]), "+r"(c[20]), "+r"(c[21]), "+r"(c[22]), "+r"(c[23]),
+                   "+r"(c[24]), "+r"(c[25]), "+r"(c[26]), "+r"(c[27]), "+r"(c[28]), "+r"(c[29]), "+r"(c[30]), "+r"(c[31]) :: "memory");
+}
+__global__ void __launch_bounds__(TC_BLOCK, TC_MIN_BLOCKS) k_check_tc(const CheckArgs a) {
+    extern __shared__ __align__(16) uint32_t s_pool[];
+    __shared__ __align__(128) uint4 s_a[6 * TC_BLOCK];             // A: [16-byte K chunk][instance]
+    __shared__ __align__(128) uint4 s_b[3 * BF_BYTES / 16];         // B: the row's three byte-fold blocks
+    __shared__ __align__(8) unsigned long long s_mbar;             // completion of the row's MMAs (tcgen05.commit)
+    __shared__ uint32_t s_tmem, s_q[8];
+    for (uint32_t t = threadIdx.x; t < a.n_pool * 8; t += TC_BLOCK) s_pool[t] = a.pool[t];
+    if (threadIdx.x < 8) s_q[threadIdx.x] = c_q[threadIdx.x];
+    const uint32_t warp = threadIdx.x >> 5;
+    const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&s_mbar);
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(&s_tmem)), "r"(TC_TMEM_COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    if (threadIdx.x == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mbar) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    tc_fence_before_sync();
+    __syncthreads();
+    tc_fence_after_sync();
+    const uint32_t tmem = s_tmem;
+    QRegs q;
+#pragma unroll
+    for (int k = 0; k < 8; k++) q.v[k] = s_q[k];
+    const uint64_t i = (uint64_t)blockIdx.x * TC_BLOCK + threadIdx.x;
+    const bool valid = i < a.n_inst;                               // threads past n_inst evaluate instance 0 and count nothing
+    const uint64_t il = valid ? i : 0;
+    const uint32_t sa = (uint32_t)__cvta_generic_to_shared(s_a), sb = (uint32_t)__cvta_generic_to_shared(s_b);
+    SmemPool pool = {s_pool};
+    unsigned long long first_bad = ~0ull;
+    uint32_t bad = 0;
+    for (uint32_t r = 0; r < a.n_rows; r++) {
+        const DevRow row = a.rows[r];
+#pragma unroll
+        for (uint32_t p = 0; p < 2; p++) {                           // 192 16-byte pieces (selected, not indexed: row stays in registers)
+            const uint32_t c = threadIdx.x + p * TC_BLOCK, k = c / (BF_BYTES / 16);
+            if (c >= 3 * BF_BYTES / 16) break;
+            const uint32_t blk = k == 0 ? row.bfold[0] : k == 1 ? row.bfold[1] : row.bfold[2];
+            const uint4* src = a.bfold + blk * (BF_BYTES / 16) + c % (BF_BYTES / 16);
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sb + 16 * c), "l"(src) : "memory");
+        }
+        asm volatile("cp.async.commit_group;" ::: "memory");
+        Fr w[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) w[k] = row_load(row, k, il);
+#pragma unroll
+        for (int k = 1; k < 4; k++) {                                // b, c, d: K chunks 2k-2, 2k-1
+            s_a[(2 * k - 2) * TC_BLOCK + threadIdx.x] = make_uint4(w[k].v[0], w[k].v[1], w[k].v[2], w[k].v[3]);
+            s_a[(2 * k - 1) * TC_BLOCK + threadIdx.x] = make_uint4(w[k].v[4], w[k].v[5], w[k].v[6], w[k].v[7]);
+        }
+        asm volatile("cp.async.wait_group 0;" ::: "memory");
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the generic-proxy writes of A and B become visible to the MMA
+        tc_fence_before_sync();
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            tc_fence_after_sync();
+#pragma unroll
+            for (uint32_t k = 0; k < 3; k++)
+                tc_mma(tmem, tc_desc(sa + k * 2 * TC_A_LBO, TC_A_LBO, BF_SBO), tc_desc(sb + k * BF_BYTES, BF_LBO, BF_SBO), k);
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(mbar) : "memory");
+        }
+        const Fr u = fr_add_noreduce(fr_mul_folded(a.fold + 8 * (uint32_t)row.fold, w[1], q), pool(row.sel[1]));   // q_m*b + q_l
+        uint32_t t[9];
+        fr_dot_wide<1>(t, w, &u, q);                                 // a*u: < 2q
+        add9_fr(t, row.qc_param >= 0 ? tab_load_fr(a.param, a.param_stride, (uint32_t)row.qc_param, il) : pool(row.sel[5]));
+        if (row.pi_param >= 0) add9_fr(t, tab_load_fr(a.param, a.param_stride, (uint32_t)row.pi_param, il));
+        else if (row.pi_sel != POOL_ZERO) add9_fr(t, pool(row.pi_sel));
+        mbar_wait(mbar, r & 1);
+        tc_fence_after_sync();
+        uint32_t c[32];
+        tc_load_columns(c, tmem + ((warp * 32) << 16));
+        add_byte_columns(t, c);                                      // + q_r*b + q_o*c + q_4*d: < 24484*q
+        if (valid && !limbs9_is_small_multiple_of_q(t, q)) {
+            bad++;
+            const unsigned long long g = a.base_row + i * (uint64_t)a.n_rows + r;
+            if (g < first_bad) first_bad = g;
+        }
+    }
+    tc_fence_before_sync();
+    __syncthreads();
+    if (warp == 0) {
+        tc_fence_after_sync();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TC_TMEM_COLS) : "memory");
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        bad += __shfl_xor_sync(0xffffffffu, bad, o);
+        const unsigned long long other = __shfl_xor_sync(0xffffffffu, first_bad, o);
+        first_bad = other < first_bad ? other : first_bad;
+    }
+    if ((threadIdx.x & 31) == 0 && bad) {
+        atomicAdd(a.counters + CNT_UNSAT, (unsigned long long)bad);
+        atomicMin(a.counters + CNT_FIRST_BAD, first_bad);
+    }
+}
+
 // The structure-aware check as a compiled row program (layout.h SpOp, bodies.cuh SparseProgBody); same skeleton as k_check.
 // DEPTH: loads in flight per thread inside a chain (register budget: 8 registers per load).
 struct SmemQ {

@@ -51,7 +51,8 @@ struct DevRow {               // 96 bytes
     int16_t pi_param;         // >= 0: PI is param slot pi_param of the instance
     uint16_t gate;            // GATE_ARITH (q_arith = 1), GATE_RANGE (q_range = 1, q_arith = 0) or GATE_NONE (both 0)
     uint16_t fold;            // entry of the segment's fold table that belongs to q_m (fr_mul_folded's eight constants)
-    uint16_t pad[5];
+    uint16_t bfold[3];        // blocks of the segment's byte-fold table that belong to q_r, q_o, q_4 (generic mode: k_check_tc)
+    uint16_t pad[2];
     // pre-resolved device address of instance 0 of each wire value (FR: the 32-byte scalar; BIT: the 32-bit word holding the
     // bit; ZERO: 0).  The gate-check kernel adds i*32 (or i*4) and never touches the table descriptors: no per-row
     // slot*stride products on the multiplier pipe.
@@ -85,6 +86,26 @@ static_assert(sizeof(SpOp) == 16, "SpOp must stay 16 bytes");
 
 // reserved pool entries
 enum : uint16_t { POOL_ZERO = 0, POOL_ONE = 1, POOL_MINUS_ONE = 2 };
+
+// ---- byte-fold blocks (generic gate check on the tensor cores, kernels.cuh k_check_tc) ----------------------------------------
+// For a selector s (Montgomery form) F_k = s * 2^(8k) * R^-1 mod q, k = 0..31, so that for any 256-bit wire w with bytes w_k
+//     sum_k w_k * F_k == s*w*R^-1 (mod q)      (the Montgomery product fr_mul_eo(s, w) up to a multiple of q).
+// As bytes this is [w_0 .. w_31] x B with B[k][j] = byte j of F_k: a dense 32 x 32 u8 matrix, the B operand of the int8 MMA.  The
+// block is stored as the MMA reads it from shared memory: K-major, no swizzle, core matrices of 8 rows (j) x 16 bytes (k).  With
+// the core matrices of one 16-byte K chunk stacked along j, element (j, k) sits at (k / 16) * BF_LBO + j * 16 + k % 16.
+constexpr uint32_t BF_BYTES = 1024;       // one block
+constexpr uint32_t BF_LBO = 512;          // leading-dimension byte offset: from one 16-byte K chunk to the next
+constexpr uint32_t BF_SBO = 128;          // stride-dimension byte offset: from rows j..j+7 to rows j+8..j+15
+PG_HD uint32_t bf_offset(uint32_t j, uint32_t k) { return (k >> 4) * BF_LBO + j * 16 + (k & 15); }
+// the block of selector s (host: template building)
+inline void byte_fold_block(uint8_t* blk, const Fr& s) {
+    for (uint32_t k = 0; k < 32; k++) {
+        Fr p = {{0, 0, 0, 0, 0, 0, 0, 0}};
+        p.v[k >> 2] = 1u << (8 * (k & 3));                                  // 2^(8k), a plain value below q
+        const Fr f = fr_mul_cios(s, p);                                     // s * 2^(8k) * R^-1 mod q
+        for (uint32_t j = 0; j < 32; j++) blk[bf_offset(j, k)] = (uint8_t)(f.v[j >> 2] >> (8 * (j & 3)));
+    }
+}
 
 // ---- 256-bit accesses -------------------------------------------------------------------------------------------------
 // A scalar is exactly one 32-byte DRAM sector.  sm_100 has 256-bit global loads/stores (ld/st.global.v8.b32 ->
